@@ -53,7 +53,14 @@ def parse_args():
     ap.add_argument("--prop-objects", type=int, default=8)
     ap.add_argument("--no-extras", action="store_true",
                     help="skip thresholds_open / components_3d / bandwidth / gpu_eager_baseline (N = 1 only anyway)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (rank 0) as DIR/<name>.npy: labels (3-D "
+                         "components of the slab), slice_labels (stitched per-slice labels), masks_kept (per slice), "
+                         "candidate_iou / candidate_stability (scores of every AMG candidate of the last slices)")
+    args = ap.parse_args()
+    if args.dump_outputs and args.steps < 1:
+        ap.error("--dump-outputs needs --steps >= 1")
+    return args
 
 
 def workload_name(args):
@@ -514,6 +521,39 @@ def gpu_eager_baseline(args, dev):
 # ------------------------------------------------------------------------------------------------
 # B200 arm
 # ------------------------------------------------------------------------------------------------
+DUMP_BYTES = 60 << 20  # < 64 MB with the .npy headers
+
+
+def dump_outputs(path, arrays):
+    """Writes each array as path/<name>.npy, in float32 where that holds every value exactly, else float64, so that
+    two builds can be compared output for output. Above DUMP_BYTES in all, each array keeps the same share of its
+    flattened elements, picked by a fixed seed (identical positions from run to run for the same shapes)."""
+    import numpy as np
+    out = {}
+    for name, a in arrays.items():
+        f = a.astype(np.float32)
+        out[name] = f if np.array_equal(f, a) else a.astype(np.float64)
+    total = sum(f.nbytes for f in out.values())
+    os.makedirs(path, exist_ok=True)
+    for name, f in out.items():
+        if total > DUMP_BYTES:
+            k = f.size * DUMP_BYTES // total
+            f = f.reshape(-1)[np.sort(np.random.default_rng(0).choice(f.size, k, replace=False))]
+        np.save(os.path.join(path, name + ".npy"), f)
+
+
+def candidate_scores(seg, S, hw):
+    """Predicted IoU and stability score of every AMG candidate (all crops, prompts and multimask outputs) of the last
+    step's slices, as their mask generators' workspaces hold them after the step: slice j of a step runs on slice
+    worker j % nw, so the last nw slices are still there. With random-init weights at the default thresholds no
+    candidate is kept, and these scores are the only non-zero results of the step."""
+    import numpy as np
+    nw = min(seg.slice_workers, S)
+    rows = [seg._peers[j % nw].adapter._amg().base_generator._ws[tuple(hw)] for j in range(S - nw, S)]
+    return {"candidate_iou": np.stack([ws["iou"].cpu().numpy() for ws in rows]),
+            "candidate_stability": np.stack([ws["stab"].cpu().numpy() for ws in rows])}
+
+
 def run_b200(args):
     import numpy as np
     import torch
@@ -588,11 +628,16 @@ def run_b200(args):
     e0.record()
     for i in range(args.steps):
         flush.zero_()  # L2 flush between timed iterations (plus inputs/activations >> L2)
-        counts, _ = step(args.warmup + i)
+        counts, comps = step(args.warmup + i)
         kept += sum(counts)
     e1.record()
     sync_all()
     ms = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"labels": comps.cpu().numpy().view(np.uint32),
+                                         "slice_labels": labels.cpu().numpy().view(np.uint16),
+                                         "masks_kept": np.array(counts),
+                                         **candidate_scores(seg, S, labels.shape[1:])})
     launches = ops.launch_count - launches0
     t = torch.tensor([ms], dtype=torch.float64, device=dev)
     if world > 1:

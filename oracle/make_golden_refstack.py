@@ -1,4 +1,4 @@
-"""Generates tests/golden/refstack_*.npz by running the reference's OWN, UNMODIFIED hot-path Python in the build container
+"""Generates tests/golden/refstack_*.npz by running the reference's OWN, UNMODIFIED hot-path Python
 (``oracle/refstack.py`` supplies stubs for its absent third-party imports):
 
   refstack_adapter_replay.npz — ``saber.adapters.sam2.SAM2Adapter.{set_volume, segment_volume}`` (REF adapters/sam2/
@@ -11,7 +11,7 @@
       propagation.py:41-189) with ``get_adapter`` returning ``refstack.FakeAdapter``: outputs + the log of adapter calls.
       The GPU tests run the twins (``saber_b200.segmenters``) behind the same fake adapter and must reproduce both.
 
-Run in the build container only:  python -m oracle.make_golden_refstack
+Run with SABER_REFERENCE_DIR pointing at a checkout of the original SABER project:  python -m oracle.make_golden_refstack
 """
 from __future__ import annotations
 

@@ -1,8 +1,8 @@
 """Boundary / parity chain for the SABER-owned Python of the hot path (SURVEY 8a R5-R7, R9, R12):
 
-  reference's own code (run in the build container by oracle/make_golden_refstack.py, fixtures committed)
+  reference's own code (run by oracle/make_golden_refstack.py, fixtures committed)
       == oracle restatement (oracle/saber_ref.py)            -- CPU tests below, anywhere
-      == the unmodified reference re-run live                 -- CPU tests below, when /root/reference is present
+      == the unmodified reference re-run live                 -- CPU tests below, when SABER_REFERENCE_DIR is set
       == saber_b200 twins behind the same fake adapter        -- GPU tests below (the twins have no CPU path)
 
 The twin adapter itself is tied to the restatement on the GPU "given identical logits" (tests/test_gpu_video.py).
@@ -49,7 +49,7 @@ def test_oracle_adapter_restatement_matches_reference_golden(golden_dir, case):
     assert int(g[f"{name}_maskmem_rows"]) == 2  # REF predictor.py:31-34 truncated the parameter to num_maskmem rows
 
 
-@pytest.mark.skipif(not refstack.available(), reason="/root/reference is only present in the build container")
+@pytest.mark.skipif(not refstack.available(), reason="needs SABER_REFERENCE_DIR: a checkout of the original SABER project")
 def test_reference_stack_live_equals_committed_goldens(golden_dir, tmp_path, monkeypatch):
     """Re-runs oracle/make_golden_refstack.py (the unmodified reference Python) and compares with the committed files:
     the fixtures are what the reference produces, not what this repo wishes it produced."""
