@@ -80,38 +80,27 @@ int sb_attention_few_keys(const void* q, long long q_ld, const float* q_add, con
                           void* stream);
 /* Fused TwoWayAttentionBlock step 4 (sam2/modeling/sam/transformer.py: `keys = norm4(keys + cross_attn_image_to_token(
  * q=keys+key_pe, k=queries+query_pe, v=queries))`) for prompts with <= 8 tokens. sb_i2t_fold folds the q / out
- * projections into per-prompt operands (kts [B,8,128], w1t [B,64,256] (nullable), w2t [B,256,64], all bf16) from the
- * projected token keys / values kt, vt [B*nt,128] bf16 (bo != NULL folds the out-projection bias into w2t: only for
- * sb_i2t_block_tc); sb_i2t_block then makes one pass over the image stream
- * x [B*nq,256] bf16 (or [nq,256] when x_shared): scores, per-head softmax, out projection, residual, LayerNorm.
- * qp [nq,128] bf16 is shared by all prompts: the positional term image_pe Wq^T + bq (w1t != NULL) or the whole query
- * projection of a shared stream (w1t == NULL). out [B*nq,256] bf16 may alias a per-prompt x. */
+ * projections and the out-projection bias bo [256] fp32 into per-prompt operands (kts [B,8,128], w1t [B,64,256],
+ * w2t [B,256,64], all bf16) from the projected token keys / values kt, vt [B*nt,128] bf16; sb_i2t_block_tc then makes
+ * one pass over the image stream x [B*nq,256] bf16 (or [nq,256] when x_shared) on tcgen05 / TMEM / TMA (128-row tiles,
+ * both GEMMs as UMMA, softmax + LayerNorm in the epilogue warps): scores, per-head softmax, out projection, residual,
+ * LayerNorm. qres [nq,128] bf16 = image_pe Wq^T + bq is shared by all prompts. out [B*nq,256] bf16 may alias a
+ * per-prompt x. */
 int sb_i2t_fold(const void* kt, long long kt_ld, const void* vt, long long vt_ld, const void* wq, const void* wo,
                 const float* bo, void* w1t, void* w2t, void* kts, int batch, int nt, float scale, void* stream);
-/* sb_i2t_block for a per-prompt stream on tcgen05 / TMEM / TMA (128-row tiles, both GEMMs as UMMA, softmax + LayerNorm in
- * the epilogue warps); w2t must carry the folded out-projection bias (sb_i2t_fold with bo != NULL). */
 int sb_i2t_block_tc(const void* x, int x_shared, const void* qres, const void* w1t, const void* w2t, const void* kts,
                     const float* gamma, const float* beta, float eps, void* out, int batch, int nq, int nt, void* stream);
-int sb_i2t_block(const void* x, int x_shared, const void* qp, const void* w1t, const void* w2t, const void* kts,
-                 const float* bo, const float* gamma, const float* beta, float eps, void* out, int batch, int nq, int nt,
-                 void* stream);
 /* Mask-decoder "tokens attend to image" (TwoWayAttentionBlock step 2, final_attn_token_to_image) for prompts with <= 8
  * tokens, computed straight on the image stream x [batch*nk (nk when x_shared), 256] bf16 without materialising K / V:
  * the k / v projections (wk, wv [128,256] bf16, bv [128] fp32; kadd [nk,128] bf16 = image_pe Wk^T + bk) fold onto the
  * token side. q [batch*nt,128] bf16 are the projected token queries; out [batch*nt,128] bf16 is the attention output
- * before out_proj. Caller-owned workspaces: qf [batch,64,256] bf16, qs [batch,8,128] bf16,
- * opart [batch,ns,64,256] fp32, ml [batch,ns,2,64] fp32 with ns = sb_t2i_fold_splits(batch, nk). */
-int sb_t2i_fold_splits(int batch, int nk);
-/* The same attention on tcgen05 / TMEM / TMA (csrc/decoder_t2i_tc.cu): QK^T and PV as M = 64 UMMAs, the TMA-staged key
- * tile is the K-major B operand of QK^T and the MN-major B operand of PV. Workspaces as above except
- * qf [batch,64,384] bf16 and ns = sb_t2i_tc_splits(batch, nk). */
+ * before out_proj. Runs on tcgen05 / TMEM / TMA (csrc/decoder_t2i_tc.cu): QK^T and PV as M = 64 UMMAs, the TMA-staged key
+ * tile is the K-major B operand of QK^T and the MN-major B operand of PV. Caller-owned workspaces: qf [batch,64,384]
+ * bf16, qs [batch,8,128] bf16, opart [batch,ns,64,256] fp32, ml [batch,ns,2,64] fp32 with ns = sb_t2i_tc_splits(batch, nk). */
 int sb_t2i_tc_splits(int batch, int nk);
 int sb_t2i_fold_attention_tc(const void* q, long long q_ld, const void* x, int x_shared, const void* kadd, const void* wk,
                              const void* wv, const float* bv, void* qf, void* qs, float* opart, float* ml, void* out,
                              long long out_ld, int batch, int nt, int nk, float scale, void* stream);
-int sb_t2i_fold_attention(const void* q, long long q_ld, const void* x, int x_shared, const void* kadd, const void* wk,
-                          const void* wv, const float* bv, void* qf, void* qs, float* opart, float* ml, void* out,
-                          long long out_ld, int batch, int nt, int nk, float scale, void* stream);
 /* Hiera MultiScaleAttention over a fused qkv buffer [B*H*W, 3*heads*hd]: window partition (with upstream's zero
  * padding of ragged windows), optional 2x2 max-pool of q, SDPA, window unpartition — hieradet.py
  * MultiScaleBlock.forward / MultiScaleAttention.forward. ws >= max(H,W) = global attention. */

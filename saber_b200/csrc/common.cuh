@@ -136,10 +136,6 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
 __device__ __forceinline__ void tma_prefetch_desc(const CUtensorMap* m) {
   asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(m)) : "memory");
 }
-// Bulk prefetch of `bytes` contiguous bytes (multiple of 16, 16-byte aligned) into L2: no destination, no completion
-__device__ __forceinline__ void prefetch_l2_bulk(const void* gptr, uint32_t bytes) {
-  asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(gptr), "r"(bytes) : "memory");
-}
 // 2-D tile load: coordinates (c0 = inner/column element index, c1 = row index)
 __device__ __forceinline__ void tma_load_2d(void* smem_dst, const CUtensorMap* m, uint64_t* bar,
                                             int32_t c0, int32_t c1) {

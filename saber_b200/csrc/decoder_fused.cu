@@ -1,6 +1,7 @@
-// saber_b200 — fused "image attends to tokens" block of the SAM2 mask decoder's two-way transformer.
+// saber_b200 — per-prompt operand fold and key-split merge of the SAM2 mask decoder's fused attention blocks, shared by
+// the two tcgen05 kernels (decoder_i2t_tc.cu, decoder_t2i_tc.cu).
 //
-// Upstream (sam2/modeling/sam/transformer.py TwoWayAttentionBlock.forward, step 4):
+// "Image attends to tokens" (upstream sam2/modeling/sam/transformer.py TwoWayAttentionBlock.forward, step 4):
 //     q = keys + key_pe ; k = queries + query_pe ; v = queries
 //     attn_out = cross_attn_image_to_token(q, k, v)          # 8 heads x 16, 4096 image queries, <= 8 token keys
 //     keys = norm4(keys + attn_out)
@@ -11,42 +12,22 @@
 //     keys_new_i       = LN(keys_i + bo + sum_{h,t} p[i,(h,t)] (Wo_h vt_{t,h}))
 // so the whole block is   S = X W1  ->  per-head softmax over 8 tokens  ->  O = P W2  ->  + residual, LayerNorm
 // with W1 [256 x 64], W2 [64 x 256] per prompt: one read and one write of the image stream (2 x 2 MB per prompt).
-// A 16-dim head is exactly one k16 MMA step and 8 tokens exactly one n8 tile, so the block-diagonal positional term is
-// one MMA per head, and the softmax of a head lives inside one accumulator tile (quad shuffles only).
+// Every head's softmax row sums to 1, so bo / 8 added to each of the 64 (head, token) columns of W2 contributes exactly
+// bo: the block needs no separate bias. i2t_fold_kernel builds W1, W2 and the scaled token keys; sb_i2t_block_tc runs
+// the block.
 //
-// Warps are autonomous: each owns 16-row tiles of the stream with a private cp.async double buffer, computes both
-// GEMMs on mma.sync.m16n8k16 (bf16 in, fp32 accumulate), normalises in registers, writes the result over its own
-// staged tile and streams it out with 16-byte coalesced stores. The per-prompt operands are staged once per CTA.
+// "Tokens attend to image" (step 2 and final_attn_token_to_image) folds the k / v projections onto the token side:
+//     score[(h,t), j] = (Wk_h^T q_{t,h}) . x_j + q_{t,h} . kadd_{j,h}          kadd = image_pe Wk^T + bk (weights only)
+//     out[t, h]       = Wv_h (sum_j p[(h,t), j] x_j) + bv_h                    (sum_j p = 1)
+// i.e. flash attention with 64 query rows of width 256 whose keys AND values are the raw image stream x [4096, 256]:
+// the stream is read once (2 MB per prompt) instead of being projected (read 2 MB, write 2 MB) and read again.
+// i2t_fold_kernel builds the folded queries, sb_t2i_fold_attention_tc computes unnormalised partial results per key
+// split, and t2i_unfold_kernel merges the splits and applies Wv / bv.
 #include "common.cuh"
 
 namespace {
 
 using bf16 = __nv_bfloat16;
-
-__device__ __forceinline__ void cp_async16(void* smem, const void* gmem) {
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(sb::smem_u32(smem)), "l"(gmem) : "memory");
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void cp_async_wait() {
-  asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory");
-}
-__device__ __forceinline__ void ldsm_x4(uint32_t addr, uint32_t& r0, uint32_t& r1, uint32_t& r2, uint32_t& r3) {
-  asm volatile("ldmatrix.sync.aligned.m8n8.x4.shared.b16 {%0,%1,%2,%3}, [%4];"
-               : "=r"(r0), "=r"(r1), "=r"(r2), "=r"(r3)
-               : "r"(addr));
-}
-__device__ __forceinline__ void ldsm_x4_trans(uint32_t addr, uint32_t& r0, uint32_t& r1, uint32_t& r2, uint32_t& r3) {
-  asm volatile("ldmatrix.sync.aligned.m8n8.x4.trans.shared.b16 {%0,%1,%2,%3}, [%4];"
-               : "=r"(r0), "=r"(r1), "=r"(r2), "=r"(r3)
-               : "r"(addr));
-}
-__device__ __forceinline__ void mma_bf16_16816(float* c, const uint32_t* a, uint32_t b0, uint32_t b1) {
-  asm volatile(
-      "mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-      : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3])
-      : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-}
 
 constexpr int I2T_C = 256;    // image stream width
 constexpr int I2T_QD = 128;   // attention width (8 heads x 16)
@@ -56,14 +37,14 @@ constexpr int I2T_NC = 64;    // (head, token) columns
 // ------------------------------------------------------------------------------------------------
 // Per-prompt folded operands. One block per prompt, 256 threads.
 //   kts [B, 8, 128]  = scale*log2(e) * kt                     (zero rows for t >= nt)
-//   w1t [B, 64, 256] : row (h*8+t), col c = scale*log2(e) * sum_d Wq[h*16+d, c] kt[t, h*16+d]      (nullable)
-//   w2t [B, 256, 64] : row c, col (h*8+t) = sum_d Wo[c, h*16+d] vt[t, h*16+d]
+//   w1t [B, 64, 256] : row (h*8+t), col c = scale*log2(e) * sum_d Wq[h*16+d, c] kt[t, h*16+d]
+//   w2t [B, 256, 64] : row c, col (h*8+t) = bo[c] / 8 + sum_d Wo[c, h*16+d] vt[t, h*16+d]      (nullable)
 // ------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256)
 i2t_fold_kernel(const bf16* __restrict__ kt, long long kt_ld, const bf16* __restrict__ vt, long long vt_ld,
                 const bf16* __restrict__ wq /* [128,256] */, const bf16* __restrict__ wo /* [256,128] */,
                 bf16* __restrict__ w1t, bf16* __restrict__ w2t, bf16* __restrict__ kts, int nt, float scale_log2,
-                const float* __restrict__ bo /* nullable: out-projection bias folded into w2t (bo / 8 per column) */,
+                const float* __restrict__ bo /* out-projection bias folded into w2t (bo / 8 per column) */,
                 int w1_ld /* row pitch of w1t (elements) */, int blockdiag /* w1t rows continue with the block-diagonal
                 scaled keys in columns [256, 384): row (h,t) holds kts[t, h*16..h*16+15] at 256 + h*16 */) {
   // One block per (head, prompt, operand): blockIdx.z == 0 -> kts + w1t (from kt), 1 -> w2t (from vt). Each thread owns
@@ -74,10 +55,8 @@ i2t_fold_kernel(const bf16* __restrict__ kt, long long kt_ld, const bf16* __rest
   const int c = tid;
   if (!second) {
     float w[16];
-    if (w1t != nullptr) {
 #pragma unroll
-      for (int d = 0; d < 16; ++d) w[d] = __bfloat162float(wq[(h * 16 + d) * I2T_C + c]);
-    }
+    for (int d = 0; d < 16; ++d) w[d] = __bfloat162float(wq[(h * 16 + d) * I2T_C + c]);
     if (tid < I2T_TOK * 16) {
       const int t = tid >> 4, d = tid & 15;
       const float v = t < nt ? __bfloat162float(kt[(static_cast<long long>(b) * nt + t) * kt_ld + h * 16 + d]) * scale_log2 : 0.f;
@@ -85,7 +64,6 @@ i2t_fold_kernel(const bf16* __restrict__ kt, long long kt_ld, const bf16* __rest
       kts[(static_cast<long long>(b) * I2T_TOK + t) * I2T_QD + h * 16 + d] = __float2bfloat16(v);
     }
     __syncthreads();
-    if (w1t == nullptr) return;
     float acc[I2T_TOK];
 #pragma unroll
     for (int t = 0; t < I2T_TOK; ++t) acc[t] = 0.f;
@@ -108,7 +86,7 @@ i2t_fold_kernel(const bf16* __restrict__ kt, long long kt_ld, const bf16* __rest
     const uint4 wa = *reinterpret_cast<const uint4*>(wo + c * I2T_QD + h * 16);
     const uint4 wb = *reinterpret_cast<const uint4*>(wo + c * I2T_QD + h * 16 + 8);
     // every head's softmax row sums to 1, so bo[c] / 8 added to all 64 (head, token) columns contributes exactly bo[c]
-    const float bfold = bo != nullptr ? bo[c] * 0.125f : 0.f;
+    const float bfold = bo[c] * 0.125f;
     if (tid < I2T_TOK * 16) {
       const int t = tid >> 4, d = tid & 15;
       sk[t][d] = t < nt ? __bfloat162float(vt[(static_cast<long long>(b) * nt + t) * vt_ld + h * 16 + d]) : 0.f;
@@ -130,437 +108,6 @@ i2t_fold_kernel(const bf16* __restrict__ kt, long long kt_ld, const bf16* __rest
     *reinterpret_cast<uint4*>(w2t + (static_cast<long long>(b) * I2T_C + c) * I2T_NC + h * 8) =
         make_uint4(sb::pack_bf16x2(acc[0], acc[1]), sb::pack_bf16x2(acc[2], acc[3]), sb::pack_bf16x2(acc[4], acc[5]),
                    sb::pack_bf16x2(acc[6], acc[7]));
-  }
-}
-
-struct I2TParams {
-  const bf16* x;           // image stream [B*nq (or nq when shared), 256]
-  long long x_bstride;     // rows between prompts (0 = one stream shared by every prompt)
-  const bf16* qp;          // [nq, 128] shared by all prompts: qres (fold mode) or the full query projection (SHARED_Q)
-  const bf16* w1t;         // [B, 64, 256] (fold mode only)
-  const bf16* w2t;         // [B, 256, 64]
-  const bf16* kts;         // [B, 8, 128]
-  const float* bo;         // [256] out-projection bias
-  const float* gamma;      // [256]
-  const float* beta;       // [256]
-  float eps;
-  bf16* out;               // [B*nq, 256]
-  int nt, nq, rows_per_cta;
-};
-
-constexpr int I2T_XP = I2T_C * 2 + 16;     // staged row pitch of the image stream / W1^T (bytes): odd multiple of 16
-constexpr int I2T_B2P = I2T_NC * 2 + 16;   // W2^T row pitch
-constexpr int I2T_KTP = I2T_QD * 2 + 32;   // token-key row pitch (8-byte fragment loads, see below)
-constexpr int I2T_WARPS = 8;
-constexpr int I2T_SMEM_X = I2T_WARPS * 2 * 16 * I2T_XP;
-constexpr int I2T_SMEM_B2 = I2T_C * I2T_B2P;
-constexpr int I2T_SMEM_KT = I2T_TOK * I2T_KTP;
-constexpr int I2T_SMEM_VEC = 3 * I2T_C * 4;
-constexpr int I2T_SMEM_B1 = I2T_NC * I2T_XP;
-constexpr int I2T_SMEM_SHARED = I2T_SMEM_X + I2T_SMEM_B2 + I2T_SMEM_KT + I2T_SMEM_VEC;
-constexpr int I2T_SMEM_FOLD = I2T_SMEM_SHARED + I2T_SMEM_B1;
-
-template <bool SHARED_Q>
-__global__ void __launch_bounds__(I2T_WARPS * 32, 1)
-i2t_block_kernel(const I2TParams p) {
-  extern __shared__ __align__(16) uint8_t smem[];
-  uint8_t* sX = smem;
-  uint8_t* sB2 = sX + I2T_SMEM_X;
-  uint8_t* sKT = sB2 + I2T_SMEM_B2;
-  float* sVec = reinterpret_cast<float*>(sKT + I2T_SMEM_KT);
-  uint8_t* sB1 = reinterpret_cast<uint8_t*>(sVec) + I2T_SMEM_VEC;
-
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const int g = lane >> 2, q4 = lane & 3;
-  const int b = blockIdx.y;
-  const int row_base = blockIdx.x * p.rows_per_cta;
-
-  // ---- per-prompt operands (one cp.async group) ----
-  {
-    const uint8_t* w2 = reinterpret_cast<const uint8_t*>(p.w2t + static_cast<long long>(b) * I2T_C * I2T_NC);
-    for (int i = tid; i < I2T_C * 8; i += I2T_WARPS * 32) cp_async16(sB2 + (i >> 3) * I2T_B2P + (i & 7) * 16, w2 + i * 16);
-    const uint8_t* kt = reinterpret_cast<const uint8_t*>(p.kts + static_cast<long long>(b) * I2T_TOK * I2T_QD);
-    for (int i = tid; i < I2T_TOK * 16; i += I2T_WARPS * 32) cp_async16(sKT + (i >> 4) * I2T_KTP + (i & 15) * 16, kt + i * 16);
-    if (!SHARED_Q) {
-      const uint8_t* w1 = reinterpret_cast<const uint8_t*>(p.w1t + static_cast<long long>(b) * I2T_NC * I2T_C);
-      for (int i = tid; i < I2T_NC * 32; i += I2T_WARPS * 32) cp_async16(sB1 + (i >> 5) * I2T_XP + (i & 31) * 16, w1 + i * 16);
-    }
-    sVec[tid] = p.bo[tid];
-    sVec[I2T_C + tid] = p.gamma[tid];
-    sVec[2 * I2T_C + tid] = p.beta[tid];
-    cp_async_commit();
-  }
-
-  const int ntiles = p.rows_per_cta / (16 * I2T_WARPS);
-  uint8_t* sXw = sX + warp * (2 * 16 * I2T_XP);
-  const bf16* xb = p.x + static_cast<long long>(b) * p.x_bstride * I2T_C;
-  auto load_tile = [&](int i, int buf) {
-    const int r0 = row_base + (i * I2T_WARPS + warp) * 16;
-    const uint8_t* src = reinterpret_cast<const uint8_t*>(xb + static_cast<long long>(r0) * I2T_C);
-    uint8_t* dst = sXw + buf * 16 * I2T_XP;
-#pragma unroll
-    for (int it = 0; it < 16; ++it) cp_async16(dst + it * I2T_XP + lane * 16, src + it * (I2T_C * 2) + lane * 16);
-  };
-  load_tile(0, 0);
-  cp_async_commit();
-  cp_async_wait<1>();
-  __syncthreads();  // the per-prompt operands are visible to every warp; from here on warps never meet again
-
-  const uint32_t b1_addr = sb::smem_u32(sB1) + ((lane & 7) + ((lane >> 4) << 3)) * I2T_XP + ((lane >> 3) & 1) * 16;
-  const uint32_t b2_addr = sb::smem_u32(sB2) + ((lane & 7) + ((lane >> 4) << 3)) * I2T_B2P + ((lane >> 3) & 1) * 16;
-  const int nt = p.nt;
-
-#pragma unroll 1
-  for (int i = 0; i < ntiles; ++i) {
-    const int buf = i & 1;
-    __syncwarp();  // every lane has finished streaming the previous tile out of the other buffer
-    if (i + 1 < ntiles) load_tile(i + 1, buf ^ 1);
-    cp_async_commit();
-    cp_async_wait<1>();
-    __syncwarp();
-    uint8_t* xt = sXw + buf * 16 * I2T_XP;
-    const uint32_t xt_s = sb::smem_u32(xt);
-    const int r0 = row_base + (i * I2T_WARPS + warp) * 16;  // first image token of this tile
-
-    // ---- S = X W1 (+ positional / shared-query term): 16 rows x 64 (head, token) columns ----
-    float s[8][4];
-#pragma unroll
-    for (int h = 0; h < 8; ++h) s[h][0] = s[h][1] = s[h][2] = s[h][3] = 0.f;
-    {
-      // one MMA per head: A = the 16 query dims of head h (straight from the shared, L2-resident [nq,128] matrix),
-      // B = the 8 token keys of head h. The k index is permuted identically on both sides (MMA k = 2*q4+e <-> dim
-      // 4*q4+e, MMA k = 8+2*q4+e <-> dim 4*q4+2+e) so that each operand is one 8-byte load per thread.
-      const bf16* q0 = p.qp + static_cast<long long>(r0 + g) * I2T_QD + q4 * 4;
-      const bf16* q1 = q0 + 8 * I2T_QD;
-      const uint8_t* kp = sKT + g * I2T_KTP + q4 * 8;
-#pragma unroll
-      for (int h = 0; h < 8; ++h) {
-        const uint2 alo = __ldg(reinterpret_cast<const uint2*>(q0 + h * 16));
-        const uint2 ahi = __ldg(reinterpret_cast<const uint2*>(q1 + h * 16));
-        const uint2 bk = *reinterpret_cast<const uint2*>(kp + h * 32);
-        const uint32_t a[4] = {alo.x, ahi.x, alo.y, ahi.y};
-        mma_bf16_16816(s[h], a, bk.x, bk.y);
-      }
-    }
-    if (!SHARED_Q) {
-      const uint32_t a_addr = xt_s + (lane & 15) * I2T_XP + (lane >> 4) * 16;
-#pragma unroll
-      for (int ks = 0; ks < 16; ++ks) {
-        uint32_t a[4];
-        ldsm_x4(a_addr + ks * 32, a[0], a[1], a[2], a[3]);
-#pragma unroll
-        for (int np = 0; np < 4; ++np) {
-          uint32_t b0, b1, b2, b3;
-          ldsm_x4(b1_addr + np * 16 * I2T_XP + ks * 32, b0, b1, b2, b3);
-          mma_bf16_16816(s[2 * np], a, b0, b1);
-          mma_bf16_16816(s[2 * np + 1], a, b2, b3);
-        }
-      }
-    }
-
-    // ---- per-head softmax over the 8 token slots (one accumulator tile per head; the quad holds a row) ----
-#pragma unroll
-    for (int h = 0; h < 8; ++h) {
-      if (2 * q4 >= nt) s[h][0] = s[h][2] = -INFINITY;
-      if (2 * q4 + 1 >= nt) s[h][1] = s[h][3] = -INFINITY;
-      float m0 = fmaxf(s[h][0], s[h][1]), m1 = fmaxf(s[h][2], s[h][3]);
-      m0 = fmaxf(m0, __shfl_xor_sync(0xffffffffu, m0, 1));
-      m1 = fmaxf(m1, __shfl_xor_sync(0xffffffffu, m1, 1));
-      m0 = fmaxf(m0, __shfl_xor_sync(0xffffffffu, m0, 2));
-      m1 = fmaxf(m1, __shfl_xor_sync(0xffffffffu, m1, 2));
-      s[h][0] = sb::fast_exp2(s[h][0] - m0);
-      s[h][1] = sb::fast_exp2(s[h][1] - m0);
-      s[h][2] = sb::fast_exp2(s[h][2] - m1);
-      s[h][3] = sb::fast_exp2(s[h][3] - m1);
-      float l0 = s[h][0] + s[h][1], l1 = s[h][2] + s[h][3];
-      l0 += __shfl_xor_sync(0xffffffffu, l0, 1);
-      l1 += __shfl_xor_sync(0xffffffffu, l1, 1);
-      l0 += __shfl_xor_sync(0xffffffffu, l0, 2);
-      l1 += __shfl_xor_sync(0xffffffffu, l1, 2);
-      const float i0 = __fdividef(1.f, l0), i1 = __fdividef(1.f, l1);
-      s[h][0] *= i0;
-      s[h][1] *= i0;
-      s[h][2] *= i1;
-      s[h][3] *= i1;
-    }
-    // accumulator tiles (2j, 2j+1) are exactly the A fragment of k16 step j of the second GEMM
-    uint32_t pa[4][4];
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      pa[j][0] = sb::pack_bf16x2(s[2 * j][0], s[2 * j][1]);
-      pa[j][1] = sb::pack_bf16x2(s[2 * j][2], s[2 * j][3]);
-      pa[j][2] = sb::pack_bf16x2(s[2 * j + 1][0], s[2 * j + 1][1]);
-      pa[j][3] = sb::pack_bf16x2(s[2 * j + 1][2], s[2 * j + 1][3]);
-    }
-
-    // ---- O = P W2: 16 rows x 256 ----
-    float o[32][4];
-#pragma unroll
-    for (int n = 0; n < 32; ++n) o[n][0] = o[n][1] = o[n][2] = o[n][3] = 0.f;
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-#pragma unroll
-      for (int np = 0; np < 16; ++np) {
-        uint32_t b0, b1, b2, b3;
-        ldsm_x4(b2_addr + np * 16 * I2T_B2P + j * 32, b0, b1, b2, b3);
-        mma_bf16_16816(o[2 * np], pa[j], b0, b1);
-        mma_bf16_16816(o[2 * np + 1], pa[j], b2, b3);
-      }
-    }
-
-    // ---- y = keys + bo + O ; LayerNorm over the 256 channels (two-pass, fp32, in registers) ----
-    float sum0 = 0.f, sum1 = 0.f;
-#pragma unroll
-    for (int n = 0; n < 32; ++n) {
-      const int c = n * 8 + 2 * q4;
-      const float2 bo2 = *reinterpret_cast<const float2*>(sVec + c);
-      const uint32_t x0 = *reinterpret_cast<const uint32_t*>(xt + g * I2T_XP + c * 2);
-      const uint32_t x1 = *reinterpret_cast<const uint32_t*>(xt + (g + 8) * I2T_XP + c * 2);
-      o[n][0] += bo2.x + sb::bf16_lo(x0);
-      o[n][1] += bo2.y + sb::bf16_hi(x0);
-      o[n][2] += bo2.x + sb::bf16_lo(x1);
-      o[n][3] += bo2.y + sb::bf16_hi(x1);
-      sum0 += o[n][0] + o[n][1];
-      sum1 += o[n][2] + o[n][3];
-    }
-    sum0 += __shfl_xor_sync(0xffffffffu, sum0, 1);
-    sum1 += __shfl_xor_sync(0xffffffffu, sum1, 1);
-    sum0 += __shfl_xor_sync(0xffffffffu, sum0, 2);
-    sum1 += __shfl_xor_sync(0xffffffffu, sum1, 2);
-    const float mean0 = sum0 * (1.f / I2T_C), mean1 = sum1 * (1.f / I2T_C);
-    float var0 = 0.f, var1 = 0.f;
-#pragma unroll
-    for (int n = 0; n < 32; ++n) {
-      const float d0 = o[n][0] - mean0, d1 = o[n][1] - mean0, d2 = o[n][2] - mean1, d3 = o[n][3] - mean1;
-      var0 = fmaf(d0, d0, fmaf(d1, d1, var0));
-      var1 = fmaf(d2, d2, fmaf(d3, d3, var1));
-    }
-    var0 += __shfl_xor_sync(0xffffffffu, var0, 1);
-    var1 += __shfl_xor_sync(0xffffffffu, var1, 1);
-    var0 += __shfl_xor_sync(0xffffffffu, var0, 2);
-    var1 += __shfl_xor_sync(0xffffffffu, var1, 2);
-    const float rstd0 = rsqrtf(var0 * (1.f / I2T_C) + p.eps), rstd1 = rsqrtf(var1 * (1.f / I2T_C) + p.eps);
-#pragma unroll
-    for (int n = 0; n < 32; ++n) {
-      const int c = n * 8 + 2 * q4;
-      const float2 ga = *reinterpret_cast<const float2*>(sVec + I2T_C + c);
-      const float2 be = *reinterpret_cast<const float2*>(sVec + 2 * I2T_C + c);
-      *reinterpret_cast<uint32_t*>(xt + g * I2T_XP + c * 2) =
-          sb::pack_bf16x2(fmaf((o[n][0] - mean0) * rstd0, ga.x, be.x), fmaf((o[n][1] - mean0) * rstd0, ga.y, be.y));
-      *reinterpret_cast<uint32_t*>(xt + (g + 8) * I2T_XP + c * 2) =
-          sb::pack_bf16x2(fmaf((o[n][2] - mean1) * rstd1, ga.x, be.x), fmaf((o[n][3] - mean1) * rstd1, ga.y, be.y));
-    }
-    __syncwarp();
-    // ---- stream the normalised tile out: one 512-byte row per warp instruction ----
-    uint8_t* dst = reinterpret_cast<uint8_t*>(p.out + (static_cast<long long>(b) * p.nq + r0) * I2T_C);
-#pragma unroll
-    for (int it = 0; it < 16; ++it)
-      *reinterpret_cast<uint4*>(dst + it * (I2T_C * 2) + lane * 16) = *reinterpret_cast<const uint4*>(xt + it * I2T_XP + lane * 16);
-  }
-  cp_async_wait<0>();
-}
-
-
-// ------------------------------------------------------------------------------------------------
-// "Tokens attend to image" (TwoWayAttentionBlock step 2 and final_attn_token_to_image) without the K|V projection of
-// the image stream. With <= 8 tokens per prompt the projections fold onto the token side:
-//     score[(h,t), j] = (Wk_h^T q_{t,h}) . x_j + q_{t,h} . kadd_{j,h}          kadd = image_pe Wk^T + bk (weights only)
-//     out[t, h]       = Wv_h (sum_j p[(h,t), j] x_j) + bv_h                    (sum_j p = 1)
-// i.e. flash attention with 64 query rows of width 256 whose keys AND values are the raw image stream x [4096, 256]:
-// the stream is read once (2 MB per prompt) instead of being projected (read 2 MB, write 2 MB) and read again.
-// CTA = (prompt, key split): 4 warps x 16 query rows (= 2 heads x 8 tokens), 32-key tiles in a 3-stage cp.async ring,
-// online softmax with lazy rescaling (the running maximum only moves when a row exceeds it by 2^8), unnormalised
-// partial results per split; t2i_unfold_kernel merges the splits and applies Wv / bv.
-// ------------------------------------------------------------------------------------------------
-constexpr int T2I_KT = 32;                          // keys per tile
-constexpr int T2I_STAGES = 3;
-constexpr int T2I_XP = I2T_C * 2 + 16;              // 528
-constexpr int T2I_KAP = I2T_QD * 2 + 16;            // 272
-constexpr int T2I_STAGE_BYTES = T2I_KT * (T2I_XP + T2I_KAP);
-constexpr int T2I_SMEM = I2T_NC * T2I_XP + T2I_STAGES * T2I_STAGE_BYTES;
-
-struct T2IParams {
-  const bf16* x;        // [B*nk (nk when shared), 256]
-  long long x_bstride;  // rows between prompts (0 = shared)
-  const bf16* kadd;     // [nk, 128]
-  const bf16* qf;       // [B, 64, 256] folded queries (scale * log2 e included)
-  const bf16* qs;       // [B, 8, 128] scaled queries
-  float* opart;         // [B, ns, 64, 256]
-  float* ml;            // [B, ns, 2, 64] (running max (log2 domain), row sum)
-  int nk, ns;
-};
-
-__global__ void __launch_bounds__(128, 2)
-t2i_fold_attn_kernel(const T2IParams p) {
-  extern __shared__ __align__(16) uint8_t smem[];
-  uint8_t* sQ = smem;
-  uint8_t* sT = smem + I2T_NC * T2I_XP;
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, g = lane >> 2, q4 = lane & 3;
-  const int b = blockIdx.y, split = blockIdx.x;
-  const int keys_per_split = p.nk / p.ns;
-  const int key0 = split * keys_per_split;
-  const int ntiles = keys_per_split / T2I_KT;
-  const bf16* xb = p.x + (static_cast<long long>(b) * p.x_bstride + key0) * I2T_C;
-  const bf16* kab = p.kadd + static_cast<long long>(key0) * I2T_QD;
-
-  auto load_tile = [&](int t) {
-    uint8_t* dx = sT + (t % T2I_STAGES) * T2I_STAGE_BYTES;
-    uint8_t* dk = dx + T2I_KT * T2I_XP;
-    const uint8_t* srcx = reinterpret_cast<const uint8_t*>(xb + static_cast<long long>(t) * T2I_KT * I2T_C);
-    const uint8_t* srck = reinterpret_cast<const uint8_t*>(kab + static_cast<long long>(t) * T2I_KT * I2T_QD);
-#pragma unroll
-    for (int i = 0; i < 8; ++i) {
-      const int c = tid + i * 128;  // 32 rows x 32 chunks
-      cp_async16(dx + (c >> 5) * T2I_XP + (c & 31) * 16, srcx + c * 16);
-    }
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      const int c = tid + i * 128;  // 32 rows x 16 chunks
-      cp_async16(dk + (c >> 4) * T2I_KAP + (c & 15) * 16, srck + c * 16);
-    }
-  };
-  {
-    const uint8_t* q = reinterpret_cast<const uint8_t*>(p.qf + static_cast<long long>(b) * I2T_NC * I2T_C);
-#pragma unroll
-    for (int i = 0; i < 16; ++i) {
-      const int c = tid + i * 128;  // 64 rows x 32 chunks
-      cp_async16(sQ + (c >> 5) * T2I_XP + (c & 31) * 16, q + c * 16);
-    }
-  }
-  load_tile(0);
-  cp_async_commit();
-  if (ntiles > 1) load_tile(1);
-  cp_async_commit();
-
-  // positional-term A fragments: this warp's rows 0-7 are head 2*warp, rows 8-15 head 2*warp+1 (token = g)
-  const int hA = 2 * warp, hB = 2 * warp + 1;
-  const bf16* qsr = p.qs + (static_cast<long long>(b) * I2T_TOK + g) * I2T_QD;
-  uint32_t aA[4], aB[4];
-  aA[0] = *reinterpret_cast<const uint32_t*>(qsr + hA * 16 + 2 * q4);
-  aA[2] = *reinterpret_cast<const uint32_t*>(qsr + hA * 16 + 8 + 2 * q4);
-  aA[1] = aA[3] = 0u;
-  aB[1] = *reinterpret_cast<const uint32_t*>(qsr + hB * 16 + 2 * q4);
-  aB[3] = *reinterpret_cast<const uint32_t*>(qsr + hB * 16 + 8 + 2 * q4);
-  aB[0] = aB[2] = 0u;
-
-  float o[32][4];
-#pragma unroll
-  for (int n = 0; n < 32; ++n) o[n][0] = o[n][1] = o[n][2] = o[n][3] = 0.f;
-  float m0 = -INFINITY, m1 = -INFINITY, l0 = 0.f, l1 = 0.f;
-
-  const uint32_t q_addr = sb::smem_u32(sQ) + (warp * 16 + (lane & 15)) * T2I_XP + (lane >> 4) * 16;
-  const uint32_t kb_off = ((lane & 7) + ((lane >> 4) << 3)) * T2I_XP + ((lane >> 3) & 1) * 16;     // QK B operand
-  const uint32_t ka_off = ((lane & 7) + ((lane >> 4) << 3)) * T2I_KAP + ((lane >> 3) & 1) * 16;    // kadd B operand
-  const uint32_t vb_off = ((lane & 7) + (((lane >> 3) & 1) << 3)) * T2I_XP + (lane >> 4) * 16;     // PV B operand (.trans)
-
-#pragma unroll 1
-  for (int t = 0; t < ntiles; ++t) {
-    cp_async_wait<1>();
-    __syncthreads();  // tile t visible to all warps; every warp is done with tile t-1 (whose stage is refilled next)
-    if (t + 2 < ntiles) load_tile(t + 2);
-    cp_async_commit();
-    const uint32_t xs = sb::smem_u32(sT + (t % T2I_STAGES) * T2I_STAGE_BYTES);
-    const uint32_t ks = xs + T2I_KT * T2I_XP;
-
-    float s[4][4];
-#pragma unroll
-    for (int n = 0; n < 4; ++n) s[n][0] = s[n][1] = s[n][2] = s[n][3] = 0.f;
-    // positional term: one k16 step per head of this warp
-#pragma unroll
-    for (int np = 0; np < 2; ++np) {
-      uint32_t b0, b1, b2, b3;
-      ldsm_x4(ks + np * 16 * T2I_KAP + ka_off + hA * 32, b0, b1, b2, b3);
-      mma_bf16_16816(s[2 * np], aA, b0, b1);
-      mma_bf16_16816(s[2 * np + 1], aA, b2, b3);
-      ldsm_x4(ks + np * 16 * T2I_KAP + ka_off + hB * 32, b0, b1, b2, b3);
-      mma_bf16_16816(s[2 * np], aB, b0, b1);
-      mma_bf16_16816(s[2 * np + 1], aB, b2, b3);
-    }
-#pragma unroll
-    for (int kk = 0; kk < 16; ++kk) {
-      uint32_t a[4];
-      ldsm_x4(q_addr + kk * 32, a[0], a[1], a[2], a[3]);
-#pragma unroll
-      for (int np = 0; np < 2; ++np) {
-        uint32_t b0, b1, b2, b3;
-        ldsm_x4(xs + np * 16 * T2I_XP + kb_off + kk * 32, b0, b1, b2, b3);
-        mma_bf16_16816(s[2 * np], a, b0, b1);
-        mma_bf16_16816(s[2 * np + 1], a, b2, b3);
-      }
-    }
-    // ---- online softmax (log2 domain; scores arrive pre-scaled) with lazy rescaling ----
-    float mx0 = fmaxf(fmaxf(s[0][0], s[0][1]), fmaxf(s[1][0], s[1][1]));
-    float mx1 = fmaxf(fmaxf(s[0][2], s[0][3]), fmaxf(s[1][2], s[1][3]));
-    mx0 = fmaxf(mx0, fmaxf(fmaxf(s[2][0], s[2][1]), fmaxf(s[3][0], s[3][1])));
-    mx1 = fmaxf(mx1, fmaxf(fmaxf(s[2][2], s[2][3]), fmaxf(s[3][2], s[3][3])));
-    mx0 = fmaxf(mx0, __shfl_xor_sync(0xffffffffu, mx0, 1));
-    mx1 = fmaxf(mx1, __shfl_xor_sync(0xffffffffu, mx1, 1));
-    mx0 = fmaxf(mx0, __shfl_xor_sync(0xffffffffu, mx0, 2));
-    mx1 = fmaxf(mx1, __shfl_xor_sync(0xffffffffu, mx1, 2));
-    if (__any_sync(0xffffffffu, (mx0 > m0 + 8.f) || (mx1 > m1 + 8.f))) {
-      const float n0 = fmaxf(m0, mx0), n1 = fmaxf(m1, mx1);
-      const float al0 = sb::fast_exp2(m0 - n0), al1 = sb::fast_exp2(m1 - n1);  // m = -inf on the first tile -> 0
-      m0 = n0;
-      m1 = n1;
-      l0 *= al0;
-      l1 *= al1;
-#pragma unroll
-      for (int n = 0; n < 32; ++n) {
-        o[n][0] *= al0;
-        o[n][1] *= al0;
-        o[n][2] *= al1;
-        o[n][3] *= al1;
-      }
-    }
-    uint32_t pa[2][4];
-#pragma unroll
-    for (int n = 0; n < 4; ++n) {
-      s[n][0] = sb::fast_exp2(s[n][0] - m0);
-      s[n][1] = sb::fast_exp2(s[n][1] - m0);
-      s[n][2] = sb::fast_exp2(s[n][2] - m1);
-      s[n][3] = sb::fast_exp2(s[n][3] - m1);
-      l0 += s[n][0] + s[n][1];
-      l1 += s[n][2] + s[n][3];
-    }
-#pragma unroll
-    for (int kk = 0; kk < 2; ++kk) {
-      pa[kk][0] = sb::pack_bf16x2(s[2 * kk][0], s[2 * kk][1]);
-      pa[kk][1] = sb::pack_bf16x2(s[2 * kk][2], s[2 * kk][3]);
-      pa[kk][2] = sb::pack_bf16x2(s[2 * kk + 1][0], s[2 * kk + 1][1]);
-      pa[kk][3] = sb::pack_bf16x2(s[2 * kk + 1][2], s[2 * kk + 1][3]);
-    }
-    // ---- O += P X (the key tile is also the value tile) ----
-#pragma unroll
-    for (int kk = 0; kk < 2; ++kk) {
-#pragma unroll
-      for (int np = 0; np < 16; ++np) {
-        uint32_t b0, b1, b2, b3;
-        ldsm_x4_trans(xs + kk * 16 * T2I_XP + vb_off + np * 32, b0, b1, b2, b3);
-        mma_bf16_16816(o[2 * np], pa[kk], b0, b1);
-        mma_bf16_16816(o[2 * np + 1], pa[kk], b2, b3);
-      }
-    }
-  }
-  cp_async_wait<0>();
-  l0 += __shfl_xor_sync(0xffffffffu, l0, 1);
-  l1 += __shfl_xor_sync(0xffffffffu, l1, 1);
-  l0 += __shfl_xor_sync(0xffffffffu, l0, 2);
-  l1 += __shfl_xor_sync(0xffffffffu, l1, 2);
-  const long long pb = static_cast<long long>(b) * p.ns + split;
-  float* op = p.opart + pb * I2T_NC * I2T_C;
-  const int r0 = warp * 16 + g, r1 = r0 + 8;
-#pragma unroll
-  for (int n = 0; n < 32; ++n) {
-    const int c = n * 8 + 2 * q4;
-    *reinterpret_cast<float2*>(op + r0 * I2T_C + c) = make_float2(o[n][0], o[n][1]);
-    *reinterpret_cast<float2*>(op + r1 * I2T_C + c) = make_float2(o[n][2], o[n][3]);
-  }
-  if (q4 == 0) {
-    float* ml = p.ml + pb * 2 * I2T_NC;
-    ml[r0] = m0;
-    ml[r1] = m1;
-    ml[I2T_NC + r0] = l0;
-    ml[I2T_NC + r1] = l1;
   }
 }
 
@@ -689,128 +236,14 @@ int sb_internal_t2i_unfold(const float* opart, const float* ml, int ns, const vo
   return SB_OK;
 }
 
-// Per-prompt folded operands of sb_i2t_block (see the header of this file). kt / vt [B*nt, 128] bf16 (the projected token
-// keys / values of cross_attn_image_to_token), wq [128,256] / wo [256,128] bf16 (its q_proj / out_proj weights).
-// w1t may be null (shared-query mode needs only kts and w2t). bo (nullable, [256] fp32): the out-projection bias is folded
-// into w2t (the tcgen05 block kernel then adds no bias); with bo == NULL w2t is the plain fold (sb_i2t_block adds bo).
+// Per-prompt folded operands of sb_i2t_block_tc (see the header of this file). kt / vt [B*nt, 128] bf16 (the projected
+// token keys / values of cross_attn_image_to_token), wq [128,256] / wo [256,128] bf16 (its q_proj / out_proj weights),
+// bo [256] fp32 (its out_proj bias, folded into w2t). Outputs: w1t [B,64,256], w2t [B,256,64], kts [B,8,128] bf16.
 extern "C" int sb_i2t_fold(const void* kt, long long kt_ld, const void* vt, long long vt_ld, const void* wq, const void* wo,
                            const float* bo, void* w1t, void* w2t, void* kts, int batch, int nt, float scale, void* stream) {
   SB_REQUIRE(batch > 0 && nt >= 1 && nt <= I2T_TOK, "sb_i2t_fold: nt must be in 1..%d (got %d)", I2T_TOK, nt);
-  SB_REQUIRE(kt && wq && kts && (w1t || w2t) && (!w2t || (vt && wo)), "sb_i2t_fold: null operand");
+  SB_REQUIRE(kt && vt && wq && wo && bo && w1t && w2t && kts, "sb_i2t_fold: null operand");
   SB_REQUIRE(((reinterpret_cast<uintptr_t>(wo) | reinterpret_cast<uintptr_t>(w2t)) & 15) == 0, "sb_i2t_fold: wo / w2t must be 16-byte aligned");
   return sb_internal_i2t_fold(kt, kt_ld, vt, vt_ld, wq, wo, bo, w1t, I2T_C, 0, w2t, kts, batch, nt, scale,
                               reinterpret_cast<cudaStream_t>(stream));
-}
-
-// keys_new = LayerNorm(keys + out_proj(softmax((keys Wq^T + qp) kt^T) vt)) for every prompt, one pass over the stream.
-// x [batch*nq, 256] bf16 (or [nq, 256] when x_shared), qp [nq, 128] bf16: the positional term of the query projection
-// (w1t != null), or the complete query projection of a stream shared by all prompts (w1t == null: layer 0 of the first
-// AMG pass). out [batch*nq, 256] bf16 (may alias x when x is per-prompt). nq must be a multiple of 256.
-extern "C" int sb_i2t_block(const void* x, int x_shared, const void* qp, const void* w1t, const void* w2t, const void* kts,
-                            const float* bo, const float* gamma, const float* beta, float eps, void* out, int batch,
-                            int nq, int nt, void* stream) {
-  SB_REQUIRE(batch > 0 && nq > 0 && (nq % 256) == 0, "sb_i2t_block: nq must be a positive multiple of 256 (got %d)", nq);
-  SB_REQUIRE(nt >= 1 && nt <= I2T_TOK, "sb_i2t_block: nt must be in 1..%d (got %d)", I2T_TOK, nt);
-  SB_REQUIRE(x && qp && w2t && kts && bo && gamma && beta && out, "sb_i2t_block: null operand");
-  SB_REQUIRE(((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(qp) | reinterpret_cast<uintptr_t>(w1t) |
-               reinterpret_cast<uintptr_t>(w2t) | reinterpret_cast<uintptr_t>(kts) | reinterpret_cast<uintptr_t>(out)) & 15) == 0,
-             "sb_i2t_block: operands must be 16-byte aligned");
-  SB_REQUIRE(!(x_shared && x == out), "sb_i2t_block: a shared stream cannot be updated in place");
-  // rows per CTA: the per-prompt operands (73 KB) are staged once per CTA, so prefer long CTAs, but keep the grid a
-  // good fit for the 148 SMs (one CTA per SM): pick the candidate with the fewest SM-waves x rows.
-  int sms = 148;
-  {
-    int dev = 0;
-    if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-  }
-  int best_rows = 256;
-  long long best_cost = -1;
-  for (int rows = 1024; rows >= 256; rows >>= 1) {
-    if (nq % rows) continue;
-    const long long ctas = static_cast<long long>(batch) * (nq / rows);
-    const long long waves = (ctas + sms - 1) / sms;
-    const long long cost = waves * (rows + 96);  // +96 rows ~ the operand staging latency of a CTA
-    if (best_cost < 0 || cost < best_cost) {
-      best_cost = cost;
-      best_rows = rows;
-    }
-  }
-  I2TParams p;
-  p.x = static_cast<const bf16*>(x);
-  p.x_bstride = x_shared ? 0 : nq;
-  p.qp = static_cast<const bf16*>(qp);
-  p.w1t = static_cast<const bf16*>(w1t);
-  p.w2t = static_cast<const bf16*>(w2t);
-  p.kts = static_cast<const bf16*>(kts);
-  p.bo = bo;
-  p.gamma = gamma;
-  p.beta = beta;
-  p.eps = eps;
-  p.out = static_cast<bf16*>(out);
-  p.nt = nt;
-  p.nq = nq;
-  p.rows_per_cta = best_rows;
-  dim3 grid(nq / best_rows, batch);
-  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  static SbPerDeviceOnce attr_once;
-  if (attr_once.need()) {
-    SB_CHECK_CUDA(cudaFuncSetAttribute(i2t_block_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, I2T_SMEM_FOLD));
-    SB_CHECK_CUDA(cudaFuncSetAttribute(i2t_block_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, I2T_SMEM_SHARED));
-    attr_once.mark();
-  }
-  if (w1t != nullptr)
-    i2t_block_kernel<false><<<grid, I2T_WARPS * 32, I2T_SMEM_FOLD, st>>>(p);
-  else
-    i2t_block_kernel<true><<<grid, I2T_WARPS * 32, I2T_SMEM_SHARED, st>>>(p);
-  SB_CHECK_LAUNCH();
-  return SB_OK;
-}
-
-// Token -> image attention of the mask decoder straight on the image stream (see t2i_fold_attn_kernel).
-// q [batch*nt, 128] bf16 (projected token queries incl. bias), x [batch*nk (nk when x_shared), 256] bf16, kadd [nk,128]
-// bf16 (= image_pe Wk^T + bk), wk / wv [128,256] bf16 (the k_proj / v_proj weights), bv [128] fp32.
-// Workspaces (caller-owned): qf [batch,64,256] bf16, qs [batch,8,128] bf16, opart [batch,ns,64,256] fp32,
-// ml [batch,ns,2,64] fp32 with ns = sb_t2i_fold_splits(batch, nk). out [batch*nt, 128] bf16 = the attention output
-// before out_proj. nt <= 8, nk a multiple of 256.
-extern "C" int sb_t2i_fold_splits(int batch, int nk) {
-  int ns = batch >= 96 ? 4 : 8;
-  while (ns > 1 && (nk % (ns * T2I_KT)) != 0) ns >>= 1;
-  return ns;
-}
-
-extern "C" int sb_t2i_fold_attention(const void* q, long long q_ld, const void* x, int x_shared, const void* kadd,
-                                     const void* wk, const void* wv, const float* bv, void* qf, void* qs, float* opart,
-                                     float* ml, void* out, long long out_ld, int batch, int nt, int nk, float scale,
-                                     void* stream) {
-  SB_REQUIRE(batch > 0 && nt >= 1 && nt <= I2T_TOK, "sb_t2i_fold_attention: nt must be in 1..%d (got %d)", I2T_TOK, nt);
-  SB_REQUIRE(nk > 0 && (nk % 256) == 0, "sb_t2i_fold_attention: nk must be a positive multiple of 256 (got %d)", nk);
-  SB_REQUIRE(q && x && kadd && wk && wv && bv && qf && qs && opart && ml && out, "sb_t2i_fold_attention: null operand");
-  SB_REQUIRE(((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(kadd) | reinterpret_cast<uintptr_t>(qf) |
-               reinterpret_cast<uintptr_t>(qs) | reinterpret_cast<uintptr_t>(wv) | reinterpret_cast<uintptr_t>(opart)) & 15) == 0,
-             "sb_t2i_fold_attention: operands must be 16-byte aligned");
-  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  const int ns = sb_t2i_fold_splits(batch, nk);
-  // folded queries: the same fold as the image->token block (W1^T rows = Wk_h^T q_{t,h}, scaled; kts = scaled q)
-  {
-    const int rc = sb_internal_i2t_fold(q, q_ld, nullptr, 0, wk, nullptr, nullptr, qf, I2T_C, 0, nullptr, qs, batch, nt, scale, st);
-    if (rc != SB_OK) return rc;
-  }
-  static SbPerDeviceOnce attr_once;
-  if (attr_once.need()) {
-    SB_CHECK_CUDA(cudaFuncSetAttribute(t2i_fold_attn_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, T2I_SMEM));
-    attr_once.mark();
-  }
-  T2IParams p;
-  p.x = static_cast<const bf16*>(x);
-  p.x_bstride = x_shared ? 0 : nk;
-  p.kadd = static_cast<const bf16*>(kadd);
-  p.qf = static_cast<const bf16*>(qf);
-  p.qs = static_cast<const bf16*>(qs);
-  p.opart = opart;
-  p.ml = ml;
-  p.nk = nk;
-  p.ns = ns;
-  t2i_fold_attn_kernel<<<dim3(ns, batch), 128, T2I_SMEM, st>>>(p);
-  SB_CHECK_LAUNCH();
-  return sb_internal_t2i_unfold(opart, ml, ns, wv, bv, out, out_ld, batch, nt, st);
 }

@@ -1,17 +1,18 @@
 // saber_b200 — the fused "image attends to tokens" block of the SAM2 mask decoder on tcgen05 / TMEM / TMA.
 //
-// Same math as i2t_block_kernel (decoder_fused.cu; upstream sam2/modeling/sam/transformer.py TwoWayAttentionBlock
-// step 4: keys = norm4(keys + cross_attn_image_to_token(keys + pe, tokens + pe, tokens))) with the per-prompt folded
-// operands W1 [256 x 64], W2 [64 x 256] (+ out-projection bias folded into W2: every softmax row sums to 1 per head):
+// Upstream sam2/modeling/sam/transformer.py TwoWayAttentionBlock step 4:
+// keys = norm4(keys + cross_attn_image_to_token(keys + pe, tokens + pe, tokens)), computed in one pass over the image
+// stream with the per-prompt folded operands W1 [256 x 64], W2 [64 x 256] of decoder_fused.cu (the out-projection bias
+// is folded into W2: every softmax row sums to 1 per head):
 //     S = X W1 + qres . kts      (128-row tile: tcgen05.mma M128 N64 K256, accumulator in TMEM; the block-diagonal
 //                                  positional term is 8 mma.sync steps per warp, added in registers)
 //     P = per-head softmax(S)    (one thread per (row, column half); written to shared memory as the K-major,
 //                                  128B-swizzled A operand of the second MMA)
 //     O = P W2                   (tcgen05.mma M128 N256 K64, accumulator in TMEM)
 //     keys_new = LN(X + O)       (two passes over TMEM; the residual is read from the TMA-staged X tile)
-// The mma.sync version re-reads W1 / W2 from shared memory for every 16 rows (8x the operand traffic of a 128-row
-// UMMA) and is shared-memory / latency bound at ~2.2 TB/s of HBM traffic; here the operands are read once per tile by
-// the tensor core and the SM's LSU bandwidth is left to the softmax / LayerNorm epilogue.
+// Both GEMMs run on the tensor core so that W1 / W2 are read once per 128-row tile (an earlier mma.sync kernel re-read
+// them from shared memory for every 16 rows and was shared-memory / latency bound at ~2.2 TB/s of HBM traffic); the
+// SM's LSU bandwidth is left to the softmax / LayerNorm epilogue.
 //
 // CTA = one prompt x `tiles` consecutive 128-row tiles. Warp roles: warp 0 TMA producer (W1, W2 once; X tiles into a
 // 2-deep ring), warp 1 MMA issuer, warp 2 TMEM allocator, warps 4-11 epilogue (thread = row x column half).
@@ -387,9 +388,10 @@ i2t_tc_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ C
 
 }  // namespace
 
-// tcgen05 version of sb_i2t_block (fold mode): x [batch*nq, 256] bf16 (or [nq, 256] shared by all prompts), qres [nq,128] bf16,
-// w1t [batch,64,256], w2t [batch,256,64] (out-projection bias folded in: sb_i2t_fold with bo != NULL), kts [batch,8,128].
-// out [batch*nq, 256] bf16 may alias x. nq must be a multiple of 256.
+// keys_new = LayerNorm(keys + out_proj(softmax((keys Wq^T + qres) kt^T) vt)) for every prompt, one pass over the stream.
+// x [batch*nq, 256] bf16 (or [nq, 256] shared by all prompts), qres [nq,128] bf16 (= image_pe Wq^T + bq), w1t
+// [batch,64,256], w2t [batch,256,64] (out-projection bias folded in), kts [batch,8,128]: the outputs of sb_i2t_fold.
+// out [batch*nq, 256] bf16 may alias x when x is per-prompt. nq must be a multiple of 256.
 extern "C" int sb_i2t_block_tc(const void* x, int x_shared, const void* qres, const void* w1t, const void* w2t,
                                const void* kts, const float* gamma, const float* beta, float eps, void* out, int batch,
                                int nq, int nt, void* stream) {

@@ -1,13 +1,12 @@
 // saber_b200 — mask-decoder "tokens attend to image" attention on tcgen05 / TMEM / TMA.
 //
-// Same math as t2i_fold_attn_kernel (decoder_fused.cu; upstream sam2/modeling/sam/transformer.py
-// TwoWayAttentionBlock step 2 and final_attn_token_to_image with the k / v projections folded onto the <= 8 tokens):
-// flash attention with 64 query rows (8 heads x 8 token slots) whose keys AND values are the raw image stream
-// x [4096, 256] of the prompt:
+// Upstream sam2/modeling/sam/transformer.py TwoWayAttentionBlock step 2 and final_attn_token_to_image, with the k / v
+// projections folded onto the <= 8 tokens (decoder_fused.cu): flash attention with 64 query rows (8 heads x 8 token
+// slots) whose keys AND values are the raw image stream x [4096, 256] of the prompt:
 //     S = Q'' [x | kadd]^T     Q'' = [Wk_h^T q_{t,h} | block-diagonal q_{t,h}]  (64 x 384),  kadd = image_pe Wk^T + bk
 //     O = softmax(S) x         (the value projection Wv / bv is applied afterwards on the 64 x 256 result)
-// The mma.sync version is bound by the legacy tensor path (54 % of its 0.5 MMA/clk/SM) and by shared-memory operand
-// re-reads (every warp re-loads the key tile); here both GEMMs are UMMAs with M = 64:
+// Both GEMMs are UMMAs with M = 64 (an earlier mma.sync kernel was bound by the legacy tensor path, 54 % of its
+// 0.5 MMA/clk/SM, and by every warp re-loading the key tile from shared memory):
 //   * QK^T: A = Q'' (K-major, resident), B = the TMA-staged key tile [64 keys x (256 + 128)] (K-major), D = S in TMEM
 //   * PV  : A = P (bf16, written by the softmax warps as a K-major 128B-swizzled tile), B = the SAME key tile read as
 //           an MN-major operand (N = 256 channels contiguous, K = keys), D = O in TMEM (fp32, 64 x 256)
@@ -303,9 +302,12 @@ extern "C" int sb_t2i_tc_splits(int batch, int nk) {
   return ns;
 }
 
-// tcgen05 version of sb_t2i_fold_attention. Same operands; workspaces: qf [batch,64,384] bf16 (folded queries followed by
-// the block-diagonal scaled queries), qs [batch,8,128] bf16, opart [batch,ns,64,256] fp32, ml [batch,ns,2,64] fp32 with
-// ns = sb_t2i_tc_splits(batch, nk).
+// Token -> image attention of the mask decoder straight on the image stream (see the header of this file).
+// q [batch*nt, 128] bf16 (projected token queries incl. bias), x [batch*nk (nk when x_shared), 256] bf16, kadd [nk,128]
+// bf16 (= image_pe Wk^T + bk), wk / wv [128,256] bf16 (the k_proj / v_proj weights), bv [128] fp32. Workspaces
+// (caller-owned): qf [batch,64,384] bf16 (folded queries followed by the block-diagonal scaled queries), qs [batch,8,128]
+// bf16, opart [batch,ns,64,256] fp32, ml [batch,ns,2,64] fp32 with ns = sb_t2i_tc_splits(batch, nk).
+// out [batch*nt, 128] bf16 = the attention output before out_proj. nt <= 8, nk a multiple of 256.
 extern "C" int sb_t2i_fold_attention_tc(const void* q, long long q_ld, const void* x, int x_shared, const void* kadd,
                                         const void* wk, const void* wv, const float* bv, void* qf, void* qs, float* opart,
                                         float* ml, void* out, long long out_ld, int batch, int nt, int nk, float scale,

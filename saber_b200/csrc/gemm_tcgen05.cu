@@ -19,10 +19,6 @@
 // drains stage s, so two tile epilogues (the bottleneck of the small-K, HBM-bound GEMMs of this model) run
 // concurrently and overlap the main loop of the following tiles. Inside an epilogue the TMEM load and the residual
 // loads of column chunk c+1 are issued before chunk c is processed.
-// An optional variant of the two up-scaling epilogues (UP1 / UP2) runs SIXTEEN epilogue warps (640 threads): every tile
-// is drained by four sets at once, set q taking the q-th of the four d-groups of the transposed convolution (64 resp.
-// 32 accumulator columns). It was built on the hypothesis that 8 warps cannot fill the issue slots; measured, it is 10 %
-// slower (same instruction count, more barriers), so it is opt-in (SB_UP_WARPS=16) and kept for A/B measurements.
 #include "common.cuh"
 #include <stdlib.h>
 
@@ -31,7 +27,7 @@ namespace {
 constexpr int BM = 128;
 constexpr int BK = 64;  // 64 bf16 = 128 B = one swizzle row
 constexpr int CH = 16;  // epilogue column chunk
-constexpr int NTHREADS = 384;   // 8 epilogue warps; the EW = 16 variants run 640 threads
+constexpr int NTHREADS = 384;   // 4 role warps + 8 epilogue warps
 
 enum { EPI_STD = 0, EPI_LN = 1, EPI_UP1 = 2, EPI_UP2 = 3 };
 
@@ -649,7 +645,7 @@ __device__ __forceinline__ void epilogue_up1(const GemmParams& p, const EpiSmem&
 
 // ---- UP2 epilogue: N = 4 groups x 32 channels -> 4 mask logits per output pixel --------------------------
 __device__ __forceinline__ void epilogue_up2(const GemmParams& p, const EpiSmem& es, uint32_t tmem_acc, int m_idx,
-                                             int q, int lane, int d_begin, int d_end, int hy_off = 256) {
+                                             int q, int lane, int d_begin, int d_end, int hy_off) {
   const int row = m_idx + q * 32 + lane;
   const bool row_ok = row < p.M;
   const uint32_t taddr = tmem_acc + (static_cast<uint32_t>(q * 32) << 16);
@@ -714,13 +710,11 @@ __device__ __forceinline__ void epilogue_up2(const GemmParams& p, const EpiSmem&
   }
 }
 
-template <int BN, int EPI, int ACT, int EW>
-__global__ void __launch_bounds__((4 + EW) * 32, 1)
+template <int BN, int EPI, int ACT>
+__global__ void __launch_bounds__(NTHREADS, 1)
 gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
                          const GemmParams p, const int stages, const int res_bufs, const int staged,
                          const int stg_out_bytes, const int stg_res_bytes, const int split, const int vec_all_bytes) {
-  static_assert(EW == 8 || (EW == 16 && (EPI == EPI_UP1 || EPI == EPI_UP2 || (EPI == EPI_STD && (BN == 128 || BN == 256)))),
-                "16 epilogue warps: up-scaling epilogues, or STD with 128 / 256-wide tiles (column quarters)");
   using C = Cfg<BN>;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) &
@@ -762,7 +756,7 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
     }
     for (int i = 0; i < 2; ++i) {
       sb::mbar_init(&tfull_bar[i], 1);
-      sb::mbar_init(&tempty_bar[i], (EW == 16 || split) ? EW : 4);  // one arrive per warp that drains this stage
+      sb::mbar_init(&tempty_bar[i], split ? 8 : 4);  // one arrive per warp that drains this stage
     }
     sb::fence_barrier_init();
   }
@@ -777,25 +771,13 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
 
   if (warp == 0) {
     // ===================== TMA producer =====================
-    // Lane 0 feeds the operand ring. Optional experiment (SB_GEMM_PF=1, off by default: it measured slower): all 32 lanes
-    // first pull the tile's RESIDUAL rows into L2 with bulk prefetches, a tile ahead of the epilogue that gathers them.
-    const bool pf_res = EPI == EPI_STD && staged > 1 && p.res != nullptr && p.res_mod == 0;
-    const int res_esz = p.res_f32 ? 4 : 2;
+    // Lane 0 feeds the operand ring.
     int stage = 0;
     uint32_t phase = 0;
     long long prof_acc = 0;
     for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
       const int m_idx = tile_m(tile);
       const int n_idx = (tile % n_tiles) * BN;
-      if (pf_res) {
-        const uint32_t bytes = static_cast<uint32_t>(min(BN, p.N - n_idx) * res_esz);
-        for (int r = lane; r < BM; r += 32) {
-          const int row = m_idx + r;
-          if (row < p.M)
-            sb::prefetch_l2_bulk(reinterpret_cast<const uint8_t*>(p.res) +
-                                     (static_cast<long long>(row) * p.ldr + n_idx) * res_esz, bytes);
-        }
-      }
       if (lane == 0) {
         for (int kb = 0; kb < num_kb; ++kb) {
           if (p.prof) {
@@ -882,51 +864,6 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
     // ===================== epilogue: set s = (warp - 4) / 4 drains accumulator stage s =====================
     const int q = warp & 3;  // TMEM lane quadrant this warp may access
     const int set = (warp - 4) >> 2;
-    if (EW == 16 && EPI != EPI_STD) {
-      // ---- four sets drain every tile together: set `set` takes d-group `set` of the transposed convolution
-      EpiSmem es;
-      {
-        // UP1: one 4 KB tile per warp (the output staging re-uses the skip staging: the skip values are in registers
-        // before the normalised row is written); UP2: two skip tiles (this tile's and, prefetched, the next tile's are
-        // not needed: one d-group per warp and tile -> a single tile)
-        uint8_t* mine = sEpi + (warp - 4) * STG_BYTES;
-        es.out_stg = sb::smem_u32(mine);
-        es.res0 = es.res1 = sb::smem_u32(mine);
-        es.nres = 1;
-        es.alias = 0;
-      }
-      const int tid512 = (warp - 4) * 32 + lane;
-      int it = 0;
-      for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x, ++it) {
-        const int st = it & 1;
-        const uint32_t acc_phase = static_cast<uint32_t>((it >> 1) & 1);
-        const int m_idx = tile_m(tile);
-        float* vec = sVec + st * VEC_FLOATS;
-        es.vec = sb::smem_u32(vec);
-        asm volatile("bar.sync 1, 512;" ::: "memory");  // every warp is done with the previous tiles' vectors
-        if (EPI == EPI_UP1) {
-          for (int c = tid512 * 4; c < 256; c += 2048) *reinterpret_cast<float4*>(vec + c) = __ldg(reinterpret_cast<const float4*>(p.bias + c));
-          if (tid512 < 16) *reinterpret_cast<float4*>(vec + 256 + tid512 * 4) = __ldg(reinterpret_cast<const float4*>(p.gamma + tid512 * 4));
-          else if (tid512 < 32) *reinterpret_cast<float4*>(vec + 512 + (tid512 - 16) * 4) = __ldg(reinterpret_cast<const float4*>(p.beta + (tid512 - 16) * 4));
-        } else {
-          if (tid512 < 32) *reinterpret_cast<float4*>(vec + tid512 * 4) = __ldg(reinterpret_cast<const float4*>(p.bias + tid512 * 4));
-          else if (tid512 < 64)
-            *reinterpret_cast<float4*>(vec + 256 + (tid512 - 32) * 4) =
-                __ldg(reinterpret_cast<const float4*>(p.hyper + static_cast<long long>(m_idx / (p.gh * p.gw)) * 128 + (tid512 - 32) * 4));
-        }
-        asm volatile("bar.sync 1, 512;" ::: "memory");
-        sb::mbar_wait(&tfull_bar[st], acc_phase);
-        sb::tc_fence_after();
-        const uint32_t tmem_acc = tmem_base + static_cast<uint32_t>(st * C::ACC_STRIDE);
-        if (EPI == EPI_UP1)
-          epilogue_up1(p, es, tmem_acc, m_idx, q, lane, set, set + 1);
-        else
-          epilogue_up2(p, es, tmem_acc, m_idx, q, lane, set, set + 1);
-        sb::tc_fence_before();
-        __syncwarp();
-        if (lane == 0) sb::mbar_arrive(&tempty_bar[st]);
-      }
-    } else {
     EpiSmem es;
     {
       // per warp: one output staging tile (32 rows x 128 B, or x 64 B for bf16 output of the STD / LN epilogues) and
@@ -954,12 +891,12 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
     if (vec_all) {
       const int tid256 = (warp - 4) * 32 + lane;
       const int valid = (p.N + 3) & ~3;
-      for (int c = tid256 * 4; c < vec_all_bytes / 4; c += EW * 128) {
+      for (int c = tid256 * 4; c < vec_all_bytes / 4; c += NEPI_WARPS * 128) {
         float4 b4 = make_float4(0.f, 0.f, 0.f, 0.f);
         if (p.bias != nullptr && c < valid) b4 = __ldg(reinterpret_cast<const float4*>(p.bias + c));
         *reinterpret_cast<float4*>(sVec + c) = b4;
       }
-      asm volatile("bar.sync 6, %0;" ::"n"(EW * 32) : "memory");
+      asm volatile("bar.sync 6, %0;" ::"n"(NEPI_WARPS * 32) : "memory");
     } else if (const_vec) {
       if (EPI == EPI_STD) {
         stage_vec(myvec, p.bias, BN, (p.N + 3) & ~3, tid128);
@@ -1025,7 +962,7 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
       sb::tc_fence_after();
       const uint32_t tmem_acc = tmem_base + static_cast<uint32_t>(st * C::ACC_STRIDE);
       // column range of this warp: its half of the tile (split) or all of it
-      const int part = split ? set : 0, nparts = split ? EW / 4 : 1;
+      const int part = split ? set : 0, nparts = split ? 2 : 1;
       if (EPI == EPI_STD) {
         constexpr int NG = BN / 32;
         if (staged) {
@@ -1060,7 +997,6 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
       atomicAdd(p.prof + 4, e_cnt[1]);
       atomicAdd(p.prof + 7, e_cnt[2]);
     }
-    }
   }
 
   sb::tc_fence_before();
@@ -1071,13 +1007,13 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
   }
 }
 
-template <int BN, int EPI, int ACT = 0, int EW = 8>
+template <int BN, int EPI, int ACT = 0>
 int launch_gemm(const CUtensorMap& tmA, const CUtensorMap& tmB, const GemmParams& p, int num_sms,
                 cudaStream_t stream) {
   using C = Cfg<BN>;
   static SbPerDeviceOnce attr_once;
   if (attr_once.need()) {
-    SB_CHECK_CUDA(cudaFuncSetAttribute(gemm_bf16_tcgen05_kernel<BN, EPI, ACT, EW>,
+    SB_CHECK_CUDA(cudaFuncSetAttribute(gemm_bf16_tcgen05_kernel<BN, EPI, ACT>,
                                        cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_MAX));
     attr_once.mark();
   }
@@ -1090,30 +1026,21 @@ int launch_gemm(const CUtensorMap& tmA, const CUtensorMap& tmB, const GemmParams
              (p.res_mod == 0 || (p.res_mod % 32) == 0) &&
              (static_cast<long long>(p.M) * ob < (1ll << 35)) && (!p.res || static_cast<long long>(p.M) * rb < (1ll << 35));
   }
-  // SB_GEMM_PF=1 switches the residual L2 prefetch on. Measured OFF is better (profiles/r02l_encoder_ab.log): with 128
-  // bulk-prefetch instructions per tile in front of the operand loads the proj GEMM fell from 356 to 249 TFLOP/s.
-  static int pf_env = -1;
-  if (pf_env < 0) {
-    const char* e = getenv("SB_GEMM_PF");
-    pf_env = (e && atoi(e) == 1) ? 1 : 0;
-  }
-  if (staged && pf_env) staged = 2;
   const bool needs_res = (EPI == EPI_UP1 || EPI == EPI_UP2) || (p.res != nullptr);
-  constexpr bool UPW = EW == 16 && EPI != EPI_STD;  // the up-scaling variant with 16 warps: one 4 KB staging tile per warp
-  int res_bufs = UPW ? 0 : (needs_res ? 2 : 0);
+  int res_bufs = needs_res ? 2 : 0;
   const int num_kb = (p.K + BK - 1) / BK;
-  const bool narrow = (EPI == EPI_STD || EPI == EPI_LN) && !UPW;
+  const bool narrow = EPI == EPI_STD || EPI == EPI_LN;
   const int stg_res_bytes = (narrow && p.res != nullptr && !p.res_f32) ? STG_BYTES / 2 : STG_BYTES;
   // STD with a residual of the output's element size: outputs are staged in place of the residual tile (no output tile)
   const bool alias = EPI == EPI_STD && staged && p.res != nullptr && (p.out_f32 != 0) == (p.res_f32 != 0);
   const int stg_out_bytes = alias ? 0 : ((narrow && !p.out_f32) ? STG_BYTES / 2 : STG_BYTES);
-  auto epi_bytes = [&](int rbufs) { return EW * (stg_out_bytes + rbufs * stg_res_bytes) + VEC_BYTES; };
+  auto epi_bytes = [&](int rbufs) { return NEPI_WARPS * (stg_out_bytes + rbufs * stg_res_bytes) + VEC_BYTES; };
   auto stages_for = [&](int rbufs) { return (SMEM_MAX - 1024 - BAR_BYTES - epi_bytes(rbufs)) / C::STAGE_BYTES; };
   int stages = stages_for(res_bufs);
   // trade the second residual buffer for a pipeline stage when the ring would be shallow, or when the main loop is long
   // enough (K >= 1152) to hide a one-deep residual prefetch (fc2: the MMA warp waited for operands 25 % of the time
   // with 3 stages)
-  if (!UPW && needs_res && EPI != EPI_UP2 && (stages < 3 || (p.K >= 1152 && stages_for(1) > stages))) {
+  if (needs_res && EPI != EPI_UP2 && (stages < 3 || (p.K >= 1152 && stages_for(1) > stages))) {
     res_bufs = 1;
     stages = stages_for(res_bufs);
   }
@@ -1137,17 +1064,16 @@ int launch_gemm(const CUtensorMap& tmA, const CUtensorMap& tmB, const GemmParams
   }
   // UP2 (K = 64: no main loop to hide) stays on the alternating scheme: in the bench's decoder passes the split form
   // was 25 % slower (16.2 vs 12.9 ms per slice, profiles/r02w_gemm_shapes.txt vs r02k), UP1 (K = 256) 9 % faster.
-  const int split = (EW == 8 && (EPI == EPI_UP1 || (EPI == EPI_STD && p.K >= split_min_k))) ||
-                            (EW == 16 && EPI == EPI_STD) ? 1 : 0;
+  const int split = (EPI == EPI_UP1 || (EPI == EPI_STD && p.K >= split_min_k)) ? 1 : 0;
   const int smem_bytes = 1024 + BAR_BYTES + stages * C::STAGE_BYTES + epi_bytes(res_bufs) +
                          (vec_all_bytes > VEC_BYTES ? vec_all_bytes - VEC_BYTES : 0);
   const int m_tiles = (p.M + BM - 1) / BM;
   const int n_tiles = (p.N + BN - 1) / BN;
   const int tiles = m_tiles * n_tiles;
   const int grid = tiles < num_sms ? tiles : num_sms;
-  gemm_bf16_tcgen05_kernel<BN, EPI, ACT, EW><<<grid, (4 + EW) * 32, smem_bytes, stream>>>(tmA, tmB, p, stages, res_bufs, staged,
-                                                                                           stg_out_bytes, stg_res_bytes, split,
-                                                                                           vec_all_bytes);
+  gemm_bf16_tcgen05_kernel<BN, EPI, ACT><<<grid, NTHREADS, smem_bytes, stream>>>(tmA, tmB, p, stages, res_bufs, staged,
+                                                                                stg_out_bytes, stg_res_bytes, split,
+                                                                                vec_all_bytes);
   SB_CHECK_LAUNCH();
   return SB_OK;
 }
@@ -1685,26 +1611,17 @@ extern "C" int sb_gemm_bf16(const void* A, long long lda, const void* W, long lo
   CUtensorMap tmA, tmB;
   int rc = make_maps(A, lda, W, ldw, M, N, K, bn, &tmA, &tmB);
   if (rc != SB_OK) return rc;
-#define SB_DISPATCH_ACT(BN_, EW_)                                                        \
-  switch (act) {                                                                        \
-    case 1: return launch_gemm<BN_, EPI_STD, 1, EW_>(tmA, tmB, p, g_num_sms, stream);   \
-    case 2: return launch_gemm<BN_, EPI_STD, 2, EW_>(tmA, tmB, p, g_num_sms, stream);   \
-    case 3: return launch_gemm<BN_, EPI_STD, 3, EW_>(tmA, tmB, p, g_num_sms, stream);   \
-    default: return launch_gemm<BN_, EPI_STD, 0, EW_>(tmA, tmB, p, g_num_sms, stream);  \
+#define SB_DISPATCH_ACT(BN_)                                                        \
+  switch (act) {                                                                   \
+    case 1: return launch_gemm<BN_, EPI_STD, 1>(tmA, tmB, p, g_num_sms, stream);   \
+    case 2: return launch_gemm<BN_, EPI_STD, 2>(tmA, tmB, p, g_num_sms, stream);   \
+    case 3: return launch_gemm<BN_, EPI_STD, 3>(tmA, tmB, p, g_num_sms, stream);   \
+    default: return launch_gemm<BN_, EPI_STD, 0>(tmA, tmB, p, g_num_sms, stream);  \
   }
-  // 16 epilogue warps (column quarters of every tile): SB_GEMM_EW=16 for the 128 / 256-wide tiles with enough work
-  static int ew_env = -1;
-  if (ew_env < 0) {
-    const char* e = getenv("SB_GEMM_EW");
-    ew_env = e ? atoi(e) : 8;
-  }
-  const bool wide = ew_env == 16 && (N % 16) == 0 && M >= 4096 && K >= 128;
-  if (bn == 256 && wide) { SB_DISPATCH_ACT(256, 16) }
-  if (bn == 128 && wide) { SB_DISPATCH_ACT(128, 16) }
-  if (bn == 256) { SB_DISPATCH_ACT(256, 8) }
-  if (bn == 192) { SB_DISPATCH_ACT(192, 8) }
-  if (bn == 128) { SB_DISPATCH_ACT(128, 8) }
-  SB_DISPATCH_ACT(64, 8)
+  if (bn == 256) { SB_DISPATCH_ACT(256) }
+  if (bn == 192) { SB_DISPATCH_ACT(192) }
+  if (bn == 128) { SB_DISPATCH_ACT(128) }
+  SB_DISPATCH_ACT(64)
 #undef SB_DISPATCH_ACT
 }
 
@@ -1777,15 +1694,6 @@ extern "C" int sb_gemm_upscale1(const void* A, long long lda, const void* W, lon
   CUtensorMap tmA, tmB;
   int rc = make_maps(A, lda, W, ldw, p.M, 256, 256, 256, &tmA, &tmB);
   if (rc != SB_OK) return rc;
-  // SB_UP_WARPS=16 selects the 16-warp epilogue. Measured (profiles/r02e_decoder_probe*.log): 336 vs 289 us for the
-  // 192-prompt batch — the epilogue is bound by the number of instructions the SM has to issue (ncu: issue slots),
-  // not by per-warp latency, so more warps only add barrier and staging overhead; 8 warps stay the default.
-  static int wide = -1;
-  if (wide < 0) {
-    const char* e = getenv("SB_UP_WARPS");
-    wide = (e && atoi(e) == 16) ? 1 : 0;
-  }
-  if (wide) return launch_gemm<256, EPI_UP1, 0, 16>(tmA, tmB, p, g_num_sms, stream);
   return launch_gemm<256, EPI_UP1>(tmA, tmB, p, g_num_sms, stream);
 }
 
@@ -1818,11 +1726,5 @@ extern "C" int sb_gemm_upscale2(const void* A, long long lda, const void* W, lon
   CUtensorMap tmA, tmB;
   int rc = make_maps(A, lda, W, ldw, p.M, 128, 64, 128, &tmA, &tmB);
   if (rc != SB_OK) return rc;
-  static int wide = -1;  // see sb_gemm_upscale1: 592 vs 539 us per 192-prompt batch with 16 epilogue warps
-  if (wide < 0) {
-    const char* e = getenv("SB_UP_WARPS");
-    wide = (e && atoi(e) == 16) ? 1 : 0;
-  }
-  if (wide) return launch_gemm<128, EPI_UP2, 0, 16>(tmA, tmB, p, g_num_sms, stream);
   return launch_gemm<128, EPI_UP2>(tmA, tmB, p, g_num_sms, stream);
 }

@@ -39,14 +39,9 @@ SIGNATURES = {
                     c_float, c_void_p],
     "sb_i2t_block_tc": [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_float, c_void_p, c_int,
                         c_int, c_int, c_void_p],
-    "sb_i2t_block": [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_float,
-                     c_void_p, c_int, c_int, c_int, c_void_p],
-    "sb_t2i_fold_splits": [c_int, c_int],
     "sb_t2i_tc_splits": [c_int, c_int],
     "sb_t2i_fold_attention_tc": [c_void_p, c_ll, c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                  c_void_p, c_void_p, c_void_p, c_void_p, c_ll, c_int, c_int, c_int, c_float, c_void_p],
-    "sb_t2i_fold_attention": [c_void_p, c_ll, c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
-                              c_void_p, c_void_p, c_void_p, c_ll, c_int, c_int, c_int, c_float, c_void_p],
     "sb_mask_embed_keys": [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_ll, c_void_p, c_void_p],
     "sb_window_attention": [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int,
                             c_int, c_float, c_void_p],

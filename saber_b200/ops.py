@@ -430,56 +430,33 @@ def attention_few_keys(q: torch.Tensor, q_add: Optional[torch.Tensor], k: torch.
 
 
 def i2t_fold(kt: torch.Tensor, vt: torch.Tensor, wq: torch.Tensor, wo: torch.Tensor, batch: int, nt: int,
-             with_w1: bool = True, scale: float = 0.25, bo: Optional[torch.Tensor] = None):
-    """Per-prompt folded operands of ``i2t_block`` (TwoWayAttentionBlock step 4 with <= 8 tokens per prompt):
-    kt / vt [batch*nt, 128] bf16 (row views allowed), wq [128,256] / wo [256,128] bf16 -> (w1t [B,64,256] or None,
-    w2t [B,256,64], kts [B,8,128]) bf16."""
-    _chk_cuda(kt, vt, wq, wo)
+             bo: torch.Tensor, scale: float = 0.25):
+    """Per-prompt folded operands of ``i2t_block_tc`` (TwoWayAttentionBlock step 4 with <= 8 tokens per prompt):
+    kt / vt [batch*nt, 128] bf16 (row views allowed), wq [128,256] / wo [256,128] bf16, bo [256] fp32 (the out-projection
+    bias, folded into w2t) -> (w1t [B,64,256], w2t [B,256,64], kts [B,8,128]) bf16."""
+    _chk_cuda(kt, vt, wq, wo, bo)
     assert kt.dtype == _BF16 and vt.dtype == _BF16 and wq.dtype == _BF16 and wo.dtype == _BF16
     assert kt.shape == (batch * nt, 128) and vt.shape == kt.shape and kt.stride(1) == 1 and vt.stride(1) == 1
     assert wq.shape == (128, 256) and wq.is_contiguous() and wo.shape == (256, 128) and wo.is_contiguous()
+    assert bo.dtype == _F32 and bo.is_contiguous() and bo.numel() == 256
     dev = kt.device
-    w1t = torch.empty((batch, 64, 256), dtype=_BF16, device=dev) if with_w1 else None
+    w1t = torch.empty((batch, 64, 256), dtype=_BF16, device=dev)
     w2t = torch.empty((batch, 256, 64), dtype=_BF16, device=dev)
     kts = torch.empty((batch, 8, 128), dtype=_BF16, device=dev)
     L = _lib.load()
-    assert bo is None or (bo.dtype == _F32 and bo.is_contiguous() and bo.numel() == 256 and bo.is_cuda)
     _lib.check(L.sb_i2t_fold(kt.data_ptr(), kt.stride(0), vt.data_ptr(), vt.stride(0), wq.data_ptr(), wo.data_ptr(),
-                             _ptr(bo), _ptr(w1t), w2t.data_ptr(), kts.data_ptr(), batch, nt, scale, _stream()),
+                             bo.data_ptr(), w1t.data_ptr(), w2t.data_ptr(), kts.data_ptr(), batch, nt, scale, _stream()),
                "sb_i2t_fold")
     _count()
     return w1t, w2t, kts
 
 
-def i2t_block(x: torch.Tensor, qp: torch.Tensor, w1t: Optional[torch.Tensor], w2t: torch.Tensor, kts: torch.Tensor,
-              bo: torch.Tensor, gamma: torch.Tensor, beta: torch.Tensor, eps: float, batch: int, nq: int, nt: int,
-              x_shared: bool = False, out: Optional[torch.Tensor] = None) -> torch.Tensor:
-    """keys_new = LN(keys + out_proj(attn(keys -> tokens))) in one pass over the image stream; see csrc/decoder_fused.cu.
-    x [batch*nq (nq when x_shared), 256] bf16, qp [nq,128] bf16; ``out`` may be ``x`` itself for a per-prompt stream."""
-    _chk_cuda(x, qp, w1t, w2t, kts, bo, gamma, beta)
-    assert x.dtype == _BF16 and x.is_contiguous() and x.shape == ((1 if x_shared else batch) * nq, 256)
-    assert qp.dtype == _BF16 and qp.is_contiguous() and qp.shape == (nq, 128)
-    assert w1t is None or (w1t.dtype == _BF16 and w1t.is_contiguous() and w1t.shape == (batch, 64, 256))
-    assert w2t.dtype == _BF16 and w2t.is_contiguous() and w2t.shape == (batch, 256, 64)
-    assert kts.dtype == _BF16 and kts.is_contiguous() and kts.shape == (batch, 8, 128)
-    for v in (bo, gamma, beta):
-        assert v.dtype == _F32 and v.is_contiguous() and v.numel() == 256
-    if out is None:
-        out = torch.empty((batch * nq, 256), dtype=_BF16, device=x.device)
-    assert out.dtype == _BF16 and out.is_contiguous() and out.shape == (batch * nq, 256)
-    L = _lib.load()
-    _lib.check(L.sb_i2t_block(x.data_ptr(), int(x_shared), qp.data_ptr(), _ptr(w1t), w2t.data_ptr(), kts.data_ptr(),
-                              bo.data_ptr(), gamma.data_ptr(), beta.data_ptr(), eps, out.data_ptr(), batch, nq, nt,
-                              _stream()), "sb_i2t_block")
-    _count()
-    return out
-
-
 def i2t_block_tc(x: torch.Tensor, qres: torch.Tensor, w1t: torch.Tensor, w2t: torch.Tensor, kts: torch.Tensor,
                  gamma: torch.Tensor, beta: torch.Tensor, eps: float, batch: int, nq: int, nt: int,
                  out: Optional[torch.Tensor] = None, x_shared: bool = False) -> torch.Tensor:
-    """``i2t_block`` of a per-prompt stream on tcgen05 / TMEM / TMA (csrc/decoder_i2t_tc.cu); ``w2t`` must come from
-    ``i2t_fold(..., bo=out_proj_bias)``."""
+    """keys_new = LN(keys + out_proj(attn(keys -> tokens))) in one pass over the image stream on tcgen05 / TMEM / TMA
+    (csrc/decoder_i2t_tc.cu). x [batch*nq (nq when x_shared), 256] bf16, qres [nq,128] bf16 (= image_pe Wq^T + bq),
+    w1t / w2t / kts from ``i2t_fold``; ``out`` may be ``x`` itself for a per-prompt stream."""
     _chk_cuda(x, qres, w1t, w2t, kts, gamma, beta)
     assert x.dtype == _BF16 and x.is_contiguous() and x.shape == ((1 if x_shared else batch) * nq, 256)
     assert qres.dtype == _BF16 and qres.is_contiguous() and qres.shape == (nq, 128)
@@ -501,10 +478,11 @@ def i2t_block_tc(x: torch.Tensor, qres: torch.Tensor, w1t: torch.Tensor, w2t: to
 
 def t2i_fold_attention(q: torch.Tensor, x: torch.Tensor, kadd: torch.Tensor, wk: torch.Tensor, wv: torch.Tensor,
                        bv: torch.Tensor, batch: int, nt: int, nk: int, x_shared: bool = False,
-                       scale: float = 0.25, tc: bool = False) -> torch.Tensor:
+                       scale: float = 0.25) -> torch.Tensor:
     """Mask-decoder token -> image attention on the raw image stream (k / v projections folded onto the <= 8 tokens of a
-    prompt; csrc/decoder_fused.cu). q [batch*nt,128] bf16, x [batch*nk (nk when shared),256] bf16, kadd [nk,128] bf16,
-    wk / wv [128,256] bf16 (row views of a stacked weight allowed), bv [128] fp32 -> [batch*nt,128] bf16."""
+    prompt; both GEMMs on tcgen05, csrc/decoder_t2i_tc.cu). q [batch*nt,128] bf16, x [batch*nk (nk when shared),256]
+    bf16, kadd [nk,128] bf16, wk / wv [128,256] bf16 (row views of a stacked weight allowed), bv [128] fp32
+    -> [batch*nt,128] bf16."""
     _chk_cuda(q, x, kadd, wk, wv, bv)
     assert q.dtype == _BF16 and q.shape == (batch * nt, 128) and q.stride(1) == 1
     assert x.dtype == _BF16 and x.is_contiguous() and x.shape == ((1 if x_shared else batch) * nk, 256)
@@ -513,18 +491,17 @@ def t2i_fold_attention(q: torch.Tensor, x: torch.Tensor, kadd: torch.Tensor, wk:
         assert w_.dtype == _BF16 and w_.shape == (128, 256) and w_.is_contiguous()
     assert bv.dtype == _F32 and bv.is_contiguous() and bv.numel() == 128
     L = _lib.load()
-    ns = (L.sb_t2i_tc_splits if tc else L.sb_t2i_fold_splits)(batch, nk)
+    ns = L.sb_t2i_tc_splits(batch, nk)
     dev = q.device
-    qf = torch.empty((batch, 64, 384 if tc else 256), dtype=_BF16, device=dev)
+    qf = torch.empty((batch, 64, 384), dtype=_BF16, device=dev)
     qs = torch.empty((batch, 8, 128), dtype=_BF16, device=dev)
     opart = torch.empty((batch, ns, 64, 256), dtype=_F32, device=dev)
     ml = torch.empty((batch, ns, 2, 64), dtype=_F32, device=dev)
     out = torch.empty((batch * nt, 128), dtype=_BF16, device=dev)
-    fn = L.sb_t2i_fold_attention_tc if tc else L.sb_t2i_fold_attention  # tc: both GEMMs on tcgen05 (decoder_t2i_tc.cu)
-    _lib.check(fn(q.data_ptr(), q.stride(0), x.data_ptr(), int(x_shared), kadd.data_ptr(),
-                                       wk.data_ptr(), wv.data_ptr(), bv.data_ptr(), qf.data_ptr(), qs.data_ptr(),
-                                       opart.data_ptr(), ml.data_ptr(), out.data_ptr(), out.stride(0), batch, nt, nk, scale,
-                                       _stream()), "sb_t2i_fold_attention")
+    _lib.check(L.sb_t2i_fold_attention_tc(q.data_ptr(), q.stride(0), x.data_ptr(), int(x_shared), kadd.data_ptr(),
+                                          wk.data_ptr(), wv.data_ptr(), bv.data_ptr(), qf.data_ptr(), qs.data_ptr(),
+                                          opart.data_ptr(), ml.data_ptr(), out.data_ptr(), out.stride(0), batch, nt, nk,
+                                          scale, _stream()), "sb_t2i_fold_attention_tc")
     _count(3)
     return out
 

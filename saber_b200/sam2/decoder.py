@@ -12,7 +12,6 @@ Restates sam2/modeling/sam/{prompt_encoder,mask_decoder,transformer}.py (SURVEY 
 from __future__ import annotations
 
 import math
-import os
 from typing import Dict, Optional, Tuple
 
 import torch
@@ -41,8 +40,6 @@ class MaskDecoder:
         md, pe = "sam_mask_decoder.", "sam_prompt_encoder."
         self.dynamic_multimask_via_stability = dynamic_multimask_via_stability
         self.stab_delta, self.stab_thresh = 0.05, 0.98
-        self.t2i_tensor_core = os.environ.get("SB_T2I_TC", "1") != "0"  # tcgen05 token->image attention (0: mma.sync)
-        self.i2t_tensor_core = os.environ.get("SB_I2T_TC", "1") != "0"  # tcgen05 image->token block (0: mma.sync kernel)
 
         def w16(t):  # bf16 GEMM operand (fp32 in the validation mode)
             return ops.weight(t, dev)
@@ -216,7 +213,7 @@ class MaskDecoder:
             q = ops.gemm(ops.add_cast(queries, query_pe, _BF16), L["t2i_q_w"], L["t2i_q_b"])
             if fuse8:  # k / v projections folded onto the tokens: the image stream is read once, K|V never exist
                 a = ops.t2i_fold_attention(q, keys, L["t2i_k_add"], L["t2i_kv_w"][0:128], L["t2i_kv_w"][128:256],
-                                           L["t2i_v_b"], B, Nt, NT_IMG, x_shared=(kb == 1), tc=self.t2i_tensor_core)
+                                           L["t2i_v_b"], B, Nt, NT_IMG, x_shared=(kb == 1))
             else:
                 kv = ops.gemm(keys, L["t2i_kv_w"], L["t2i_kv_b"])
                 a = ops.attention_kadd(q, kv[:, 0:128], L["t2i_k_add"], kv[:, 128:256], B, 8, Nt, NT_IMG,
@@ -234,23 +231,13 @@ class MaskDecoder:
             # big GEMM has no residual stream to gather
             if fuse8:
                 # <= 8 tokens per prompt: q projection, attention, out projection, residual and norm4 in ONE pass over
-                # the image stream, with the projections folded into per-prompt operands (csrc/decoder_fused.cu)
-                if self.i2t_tensor_core:  # both GEMMs on tcgen05 (csrc/decoder_i2t_tc.cu); a stream shared by all
-                    # prompts (layer 0 of the first pass) is read through the same tensor map by every prompt
-                    w1t, w2t, kts = ops.i2t_fold(kt, vt, L["i2t_q_w"], L["i2t_o_w"], B, Nt, bo=L["i2t_o_b"])
-                    keys = ops.i2t_block_tc(keys, L["i2t_q_res16"], w1t, w2t, kts, L["n4w"], L["n4b"], 1e-5, B, NT_IMG, Nt,
-                                            out=(None if kb == 1 else keys), x_shared=(kb == 1))
-                    keys_f32, kb = keys, B
-                    continue
-                if kb == 1:  # one stream shared by all prompts: its query projection is computed once
-                    qp = ops.gemm(keys, L["i2t_q_w"], None, residual=L["i2t_q_res"], res_mod=NT_IMG)
-                    w1t, w2t, kts = ops.i2t_fold(kt, vt, L["i2t_q_w"], L["i2t_o_w"], B, Nt, with_w1=False)
-                else:
-                    qp = L["i2t_q_res16"]
-                    w1t, w2t, kts = ops.i2t_fold(kt, vt, L["i2t_q_w"], L["i2t_o_w"], B, Nt)
-                keys = ops.i2t_block(keys, qp, w1t, w2t, kts, L["i2t_o_b"], L["n4w"], L["n4b"], 1e-5, B, NT_IMG, Nt,
-                                     x_shared=(kb == 1), out=(None if kb == 1 else keys))  # a per-prompt stream is private to this
-                # call (built above from the image embedding): updated in place
+                # the image stream, with the projections folded into per-prompt operands (csrc/decoder_fused.cu) and
+                # both GEMMs on tcgen05 (csrc/decoder_i2t_tc.cu). A stream shared by all prompts (layer 0 of the first
+                # pass) is read through the same tensor map by every prompt; a per-prompt stream is private to this
+                # call (built above from the image embedding) and is updated in place.
+                w1t, w2t, kts = ops.i2t_fold(kt, vt, L["i2t_q_w"], L["i2t_o_w"], B, Nt, bo=L["i2t_o_b"])
+                keys = ops.i2t_block_tc(keys, L["i2t_q_res16"], w1t, w2t, kts, L["n4w"], L["n4b"], 1e-5, B, NT_IMG, Nt,
+                                        out=(None if kb == 1 else keys), x_shared=(kb == 1))
                 keys_f32, kb = keys, B
                 continue
             if Nt <= 16 and not val:
@@ -268,7 +255,7 @@ class MaskDecoder:
         q = ops.gemm(ops.add_cast(queries, query_pe, _BF16), self.fa_q_w, self.fa_q_b)
         if fuse8:
             a = ops.t2i_fold_attention(q, keys, self.fa_k_add, self.fa_kv_w[0:128], self.fa_kv_w[128:256], self.fa_v_b, B,
-                                       Nt, NT_IMG, x_shared=(kb == 1), tc=self.t2i_tensor_core)
+                                       Nt, NT_IMG, x_shared=(kb == 1))
         else:
             kv = ops.gemm(keys, self.fa_kv_w, self.fa_kv_b)
             a = ops.attention_kadd(q, kv[:, 0:128], self.fa_k_add, kv[:, 128:256], B, 8, Nt, NT_IMG, kv_shared=(kb == 1))

@@ -551,19 +551,17 @@ def t2i_case(kind, B, nt, nk, x_shared, splits, seed=12, device="cuda"):
 @pytest.mark.gpu
 @pytest.mark.parametrize("kind", ["flat", "beacon", "beacon2"])
 @pytest.mark.parametrize("B,nt,shared", [(1, 1, False), (3, 7, False), (3, 8, True), (100, 8, False), (100, 1, True)])
-@pytest.mark.parametrize("tc", [False, True])
-def test_t2i_fold(ops, kind, B, nt, shared, tc):
-    """Route: t2i_fold_attn_kernel (mma.sync, 32-key tiles) or the tcgen05 fold kernel (64-key tiles), each followed by
-    t2i_unfold_kernel, which merges the key splits. Beacons at keys 0 / nk - 1, the first / last key of every split
-    (sb_t2i_fold_splits / sb_t2i_tc_splits) and the first tile edges."""
+def test_t2i_fold(ops, kind, B, nt, shared):
+    """Route: the tcgen05 fold kernel (64-key tiles) followed by t2i_unfold_kernel, which merges the key splits.
+    Beacons at keys 0 / nk - 1, the first / last key of every split (sb_t2i_tc_splits) and the first tile edges."""
     from saber_b200 import lib
     nk = 4096
     L = lib.load()
-    splits = (L.sb_t2i_tc_splits if tc else L.sb_t2i_fold_splits)(B, nk)
+    splits = L.sb_t2i_tc_splits(B, nk)
     q, x, kadd, wk, wv, bv = t2i_case(kind, B, nt, nk, shared, splits)
-    out = ops.t2i_fold_attention(q, x, kadd, wk, wv, bv, B, nt, nk, x_shared=shared, tc=tc)
+    out = ops.t2i_fold_attention(q, x, kadd, wk, wv, bv, B, nt, nk, x_shared=shared)
     args = (q, x, kadd, wk, wv, bv, B, nt, nk, shared)
-    assert_close(out, ref_t2i(*args), ref_t2i(*args, mode="bf16"), f"t2i tc{int(tc)} {kind} B{B} nt{nt} shared{shared} ns{splits}")
+    assert_close(out, ref_t2i(*args), ref_t2i(*args, mode="bf16"), f"t2i {kind} B{B} nt{nt} shared{shared} ns{splits}")
 
 
 @pytest.mark.gpu
