@@ -200,6 +200,20 @@ int sb_amg_fill_lowres(const float* planes, const float* ious4, const int* sel, 
  * only where the mask changed. ws: ws_ctas * 32 * H * ceil(W/32) int32. */
 int sb_amg_small_regions(void* bits, const int* rows, int m, int H, int W, int max_small, int* box, int* area,
                          float* score, int* box_changed, int* ws, int ws_ctas, void* stream);
+/* Run-length encoding of the m packed masks sel[k] (sel null: k) of bits [*, H, ceil(W/32)] (bits past W ignored), for
+ * SAM2AutomaticMaskGenerator output_mode "uncompressed_rle" / "coco_rle". Counts are upstream's mask_to_rle_pytorch:
+ * column-major runs, starting with the zeros before the first set pixel (0 when pixel (0, 0) is set), at most H*W + 1
+ * per mask; H*W < 2^31. Two phases around one host read of the total:
+ *  - sb_masks_rle_size writes offsets [m+1] int64 (the counts of mask k are counts[offsets[k] .. offsets[k+1])) and
+ *    fills ws (2*m*W int32) for sb_masks_rle_counts, which writes counts [offsets[m]] int32.
+ *  - sb_masks_rle_coco_size / sb_masks_rle_coco turn those counts into pycocotools' rleToString characters: coco_offsets
+ *    [m+1] int64 and chars [coco_offsets[m]] uint8 (no terminators). */
+int sb_masks_rle_size(const void* bits, const int* sel, int m, int H, int W, int* ws, long long* offsets, void* stream);
+int sb_masks_rle_counts(const void* bits, const int* sel, int m, int H, int W, const int* ws, const long long* offsets,
+                        int* counts, void* stream);
+int sb_masks_rle_coco_size(const int* counts, const long long* offsets, int m, long long* coco_offsets, void* stream);
+int sb_masks_rle_coco(const int* counts, const long long* offsets, int m, const long long* coco_offsets,
+                      unsigned char* chars, void* stream);
 /* REF saber/segmenters/propagation.py:181-186: masks3d[mask] = idx + 1 in list order (later masks win) */
 int sb_stitch_labels(const void* bits, const int* order, int m, int H, int W, void* labels, void* stream);
 /* REF saber/segmenters/utils.py:88-131 separate_masks: 26-connected components (scipy.ndimage.label numbering),

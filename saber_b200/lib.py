@@ -84,6 +84,10 @@ SIGNATURES = {
                            c_float, c_void_p, c_void_p, c_int, c_void_p],
     "sb_amg_small_regions": [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p,
                              c_void_p, c_int, c_void_p],
+    "sb_masks_rle_size": [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p],
+    "sb_masks_rle_counts": [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p],
+    "sb_masks_rle_coco_size": [c_void_p, c_void_p, c_int, c_void_p, c_void_p],
+    "sb_masks_rle_coco": [c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p],
     "sb_box_filter": [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p],
     "sb_contrast_normalize": [c_void_p, c_void_p, c_void_p, c_void_p, c_ll, c_float, c_void_p, c_void_p],
     "sb_rgb_mix_planar": [c_void_p, c_void_p, c_int, c_ll, c_void_p, c_void_p],

@@ -902,6 +902,40 @@ def amg_small_regions(bits: torch.Tensor, rows: Optional[torch.Tensor], m: int, 
     _count()
 
 
+def masks_to_rle(bits: torch.Tensor, sel: Optional[torch.Tensor], m: int, W: int, coco: bool = False):
+    """Run-length encoding of the packed masks [*, H, ceil(W/32)] rows sel[0..m) (or the first m), on the device.
+    Returns (data, offsets) with offsets [m+1] int64: the encoding of mask k is data[offsets[k]:offsets[k+1]], int32
+    counts of upstream's mask_to_rle_pytorch, or with ``coco`` the uint8 characters of pycocotools' rleToString.
+    Reads each total back with one host synchronisation."""
+    _chk_cuda(bits, sel)
+    H, WW = bits.shape[1], bits.shape[2]
+    assert bits.dtype == _I32 and bits.is_contiguous() and WW == (W + 31) // 32
+    assert sel is None or (sel.dtype == _I32 and sel.is_contiguous() and sel.numel() >= m)
+    assert sel is not None or bits.shape[0] >= m
+    dev = bits.device
+    offsets = torch.zeros((m + 1,), dtype=torch.int64, device=dev)
+    if m == 0:
+        return torch.empty((0,), dtype=torch.uint8 if coco else _I32, device=dev), offsets
+    L = _lib.load()
+    ws = torch.empty((2 * m * W,), dtype=_I32, device=dev)
+    _lib.check(L.sb_masks_rle_size(bits.data_ptr(), _ptr(sel), m, H, W, ws.data_ptr(), offsets.data_ptr(), _stream()),
+               "sb_masks_rle_size")
+    counts = torch.empty((int(offsets[m].item()),), dtype=_I32, device=dev)
+    _lib.check(L.sb_masks_rle_counts(bits.data_ptr(), _ptr(sel), m, H, W, ws.data_ptr(), offsets.data_ptr(),
+                                     counts.data_ptr(), _stream()), "sb_masks_rle_counts")
+    _count(4)
+    if not coco:
+        return counts, offsets
+    coff = torch.zeros((m + 1,), dtype=torch.int64, device=dev)
+    _lib.check(L.sb_masks_rle_coco_size(counts.data_ptr(), offsets.data_ptr(), m, coff.data_ptr(), _stream()),
+               "sb_masks_rle_coco_size")
+    chars = torch.empty((int(coff[m].item()),), dtype=torch.uint8, device=dev)
+    _lib.check(L.sb_masks_rle_coco(counts.data_ptr(), offsets.data_ptr(), m, coff.data_ptr(), chars.data_ptr(),
+                                   _stream()), "sb_masks_rle_coco")
+    _count(3)
+    return chars, coff
+
+
 def prepare_slice(img: torch.Tensor, box: int = 500, cutoff: float = 3.0) -> torch.Tensor:
     """REF saber/utils/preprocessing.py:67-81 ``prepare`` on one [H, W] fp32 slice -> [H, W] fp32 in [0,1]
     (the three RGB channels SABER feeds SAM2 are identical copies of it)."""

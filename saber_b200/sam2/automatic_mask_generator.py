@@ -13,7 +13,9 @@ bit-packed full-frame masks; candidate lists and their lengths stay in device me
 full-resolution logits upstream materialises per batch never exist. One synchronisation at the end
 fetches the survivor count. With ``min_mask_region_area > 0`` the decoder planes are hole / sprinkle filled on the
 device before the post-processing (inside the captured graphs), and the survivors go through upstream's
-postprocess_small_regions on their packed masks, with a second synchronisation for the new count.
+postprocess_small_regions on their packed masks, with a second synchronisation for the new count. With
+``output_mode`` "uncompressed_rle" / "coco_rle" the survivors are run-length encoded on the device and only the encodings
+are copied to the host; "binary_mask" unpacks them to dense bool masks.
 """
 from __future__ import annotations
 
@@ -112,8 +114,8 @@ class SAM2AutomaticMaskGenerator:
                  multimask_output: bool = True, **kwargs) -> None:
         if (points_per_side is None) == (point_grids is None):
             raise ValueError("Exactly one of points_per_side or point_grid must be provided.")
-        if output_mode != "binary_mask":
-            raise NotImplementedError("only output_mode='binary_mask' is on SABER's path")
+        if output_mode not in ("binary_mask", "uncompressed_rle", "coco_rle"):
+            raise ValueError(f"Unknown output_mode {output_mode}.")
         self.point_grids = (build_all_layer_point_grids(points_per_side, crop_n_layers, crop_n_points_downscale_factor)
                             if point_grids is None else point_grids)
         self.predictor = SAM2ImagePredictor(model, max_hole_area=min_mask_region_area,
@@ -460,9 +462,24 @@ class SAM2AutomaticMaskGenerator:
         recs = self.records(dm)
         if dm.count == 0:
             return []
-        seg = ops.unpack_bits(dm.bits, None, dm.count, dm.hw[1]).cpu().numpy()
+        if self.output_mode == "binary_mask":
+            seg = ops.unpack_bits(dm.bits, None, dm.count, dm.hw[1]).cpu().numpy()
+        else:
+            seg = self._rle_segmentations(dm)
         for i, r in enumerate(recs):
             r["segmentation"] = seg[i]
         return [{"segmentation": r["segmentation"], "area": r["area"], "bbox": r["bbox"],
                  "predicted_iou": r["predicted_iou"], "point_coords": r["point_coords"],
                  "stability_score": r["stability_score"], "crop_box": r["crop_box"]} for r in recs]
+
+    def _rle_segmentations(self, dm: DeviceMasks) -> List[Dict[str, Any]]:
+        """Segmentations of output_mode "uncompressed_rle" (upstream mask_to_rle_pytorch) and "coco_rle" (pycocotools'
+        rleToString, which upstream's coco_encode_rle calls), run-length encoded on the device from the packed masks:
+        only the encodings are copied to the host."""
+        H, W = dm.hw
+        data, off = ops.masks_to_rle(dm.bits, None, dm.count, W, coco=self.output_mode == "coco_rle")
+        data, off = data.cpu().numpy(), off.cpu().tolist()
+        if self.output_mode == "coco_rle":
+            text = data.tobytes().decode("ascii")
+            return [{"size": [H, W], "counts": text[a:b]} for a, b in zip(off[:-1], off[1:])]
+        return [{"size": [H, W], "counts": data[a:b].tolist()} for a, b in zip(off[:-1], off[1:])]
