@@ -242,6 +242,11 @@ int sb_resize_normalize(const float* img, int H, int W, int C, const int* crops,
                         const float* mean3, const float* std3, float* out, void* stream);
 /* F.interpolate(bilinear, align_corners=False): SAM2Transforms.postprocess_masks / video-resolution logits */
 int sb_upsample_bilinear(const float* in, int N, int Hi, int Wi, int Ho, int Wo, float* out, void* stream);
+/* SAM2ImagePredictor's full-resolution output in one pass: candidate c of P*cpp takes plane [c/cpp, token] of planes
+ * [P,4,S,S] (token 1 + c%3 for cpp = 3, else sel[c] or 0), up-samples it as sb_upsample_bilinear does and writes out
+ * [P*cpp, Ho, Wo]: fp32 logits when logits != 0, else bool (value > thr). out is 16-byte aligned. */
+int sb_upsample_select(const float* planes, int P, int S, const int* sel, int cpp, int Ho, int Wo, float thr,
+                       int logits, void* out, void* stream);
 
 /* ---- z-axis propagation: memory attention / memory encoder / tracking glue (upstream sam2_video_predictor.py, ----
  * modeling/{memory_attention,memory_encoder,sam2_base}.py, reached from REF saber/adapters/sam2/predictor.py:164-202) */

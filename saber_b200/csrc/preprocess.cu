@@ -251,6 +251,88 @@ upsample_bilinear_kernel(const float* __restrict__ in, int N, int Hi, int Wi, in
   }
 }
 
+// Decoder planes -> SAM2ImagePredictor's full-resolution output in one pass, with no intermediate buffer. Candidate c
+// of P * cpp reads plane [c / cpp, token] of planes [P, 4, S, S]: token 1 + c % 3 for cpp = 3, otherwise sel[c] or 0
+// (the candidate convention of amg_mask_post / amg_fill_lowres). It is up-sampled with upsample_bilinear_kernel's
+// expression tree, so the logits are bit-identical to it, and out[c, Ho, Wo] gets the fp32 logits or the bool
+// mask (value > thr). A thread owns UPS_RUN consecutive pixels of one row over `rows` rows: its x-taps are computed
+// once and its y-taps once per row. Each row's run is stored with V-byte stores, V = gcd(row bytes, 16) (1 when that
+// is 2): every row start, and the ragged tail of Wo % UPS_RUN pixels, is then a whole number of aligned V-byte words.
+constexpr int UPS_RUN = 16;
+
+template <int V, int NB>
+__device__ __forceinline__ void store_run(unsigned char* dst, const uint32_t (&w)[NB / 4], int nbytes) {
+#pragma unroll
+  for (int b = 0; b < NB; b += V) {
+    if (b < nbytes) {
+      if constexpr (V == 16) {
+        *reinterpret_cast<uint4*>(dst + b) = make_uint4(w[b / 4], w[b / 4 + 1], w[b / 4 + 2], w[b / 4 + 3]);
+      } else if constexpr (V == 8) {
+        *reinterpret_cast<uint2*>(dst + b) = make_uint2(w[b / 4], w[b / 4 + 1]);
+      } else if constexpr (V == 4) {
+        *reinterpret_cast<uint32_t*>(dst + b) = w[b / 4];
+      } else {
+        dst[b] = static_cast<unsigned char>(w[b / 4] >> (8 * (b % 4)));
+      }
+    }
+  }
+}
+
+template <bool LOGITS, int V>
+__global__ void __launch_bounds__(256)
+upsample_select_kernel(const float* __restrict__ planes, int P, int S, const int* __restrict__ sel, int cpp, int Ho,
+                       int Wo, int rows, float thr, unsigned char* __restrict__ out) {
+  constexpr int E = LOGITS ? 4 : 1;  // output bytes per pixel
+  constexpr int NB = UPS_RUN * E;
+  const float scale_h = __fdiv_rn(static_cast<float>(S), static_cast<float>(Ho));
+  const float scale_w = __fdiv_rn(static_cast<float>(S), static_cast<float>(Wo));
+  const int runs = (Wo + UPS_RUN - 1) / UPS_RUN;
+  const int bands = (Ho + rows - 1) / rows;
+  const long long total = static_cast<long long>(P) * cpp * bands * runs;
+  for (long long t = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x; t < total;
+       t += static_cast<long long>(gridDim.x) * blockDim.x) {
+    const int run = static_cast<int>(t % runs);
+    const long long cb = t / runs;
+    const int band = static_cast<int>(cb % bands);
+    const int c = static_cast<int>(cb / bands);
+    const int p = c / cpp;
+    const int token = cpp == 3 ? 1 + c % 3 : (sel ? __ldg(sel + p) : 0);
+    const float* plane = planes + (static_cast<long long>(p) * 4 + token) * S * S;
+    const int x_begin = run * UPS_RUN;
+    int xa[UPS_RUN];
+    float lx0[UPS_RUN], lx1[UPS_RUN];
+#pragma unroll
+    for (int i = 0; i < UPS_RUN; ++i) {
+      int x1;
+      bl_src_index(scale_w, min(x_begin + i, Wo - 1), S, xa[i], x1, lx0[i], lx1[i]);  // x1 = min(xa + 1, S - 1)
+    }
+    const int nbytes = min(UPS_RUN, Wo - x_begin) * E;
+    const int y_end = min(Ho, (band + 1) * rows);
+    for (int oy = band * rows; oy < y_end; ++oy) {
+      int y0, y1;
+      float ly0, ly1;
+      bl_src_index(scale_h, oy, S, y0, y1, ly0, ly1);
+      const float* r0 = plane + y0 * S;
+      const float* r1 = plane + y1 * S;
+      uint32_t w[NB / 4];
+#pragma unroll
+      for (int i = 0; i < UPS_RUN; ++i) {
+        const int x1 = min(xa[i] + 1, S - 1);
+        const float t0 = __fmaf_rn(__ldg(r0 + xa[i]), lx0[i], __fmul_rn(__ldg(r0 + x1), lx1[i]));
+        const float t1 = __fmaf_rn(__ldg(r1 + xa[i]), lx0[i], __fmul_rn(__ldg(r1 + x1), lx1[i]));
+        const float v = __fmaf_rn(t0, ly0, __fmul_rn(t1, ly1));
+        if constexpr (LOGITS) {
+          w[i] = __float_as_uint(v);
+        } else {
+          const uint32_t bit = (v > thr ? 1u : 0u) << (8 * (i % 4));
+          w[i / 4] = (i % 4 == 0) ? bit : (w[i / 4] | bit);
+        }
+      }
+      store_run<V, NB>(out + ((static_cast<long long>(c) * Ho + oy) * Wo + x_begin) * E, w, nbytes);
+    }
+  }
+}
+
 inline int grid_for(long long total, int block = 256, int cap = 148 * 16) {
   long long g = (total + block - 1) / block;
   if (g > cap) g = cap;
@@ -369,6 +451,45 @@ extern "C" int sb_upsample_bilinear(const float* in, int N, int Hi, int Wi, int 
   SB_REQUIRE(N > 0 && Hi > 0 && Wi > 0 && Ho > 0 && Wo > 0, "sb_upsample_bilinear: bad sizes");
   const long long total = static_cast<long long>(N) * Ho * Wo;
   upsample_bilinear_kernel<<<grid_for(total, 256, 148 * 32), 256, 0, stream>>>(in, N, Hi, Wi, Ho, Wo, out);
+  SB_CHECK_LAUNCH();
+  return SB_OK;
+}
+
+// planes: [P, 4, S, S] fp32; sel: [P] int32 or null; cpp 3 (tokens 1..3) or 1 (sel, or token 0).
+// out: [P * cpp, Ho, Wo] fp32 logits (logits != 0) or bool (value > thr), 16-byte aligned.
+extern "C" int sb_upsample_select(const float* planes, int P, int S, const int* sel, int cpp, int Ho, int Wo, float thr,
+                                  int logits, void* out, void* stream_) {
+  cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
+  SB_REQUIRE(planes && out && P > 0 && S > 0 && Ho > 0 && Wo > 0 && (cpp == 1 || cpp == 3),
+             "sb_upsample_select: bad arguments");
+  SB_REQUIRE((reinterpret_cast<uintptr_t>(out) & 15) == 0, "sb_upsample_select: out must be 16-byte aligned");
+  const int E = logits ? 4 : 1;
+  int V = 16;
+  while ((static_cast<long long>(Wo) * E) % V) V >>= 1;
+  const long long cands = static_cast<long long>(P) * cpp, runs = (Wo + UPS_RUN - 1) / UPS_RUN;
+  // up to 8 rows per thread, fewer while that would leave the GPU short of threads (few candidates, small frames)
+  int rows = 8;
+  while (rows > 1 && cands * ((Ho + rows - 1) / rows) * runs < 148LL * 1024) rows >>= 1;
+  const long long total = cands * ((Ho + rows - 1) / rows) * runs;
+  const int grid = grid_for(total, 256, 148 * 32);
+  unsigned char* o = static_cast<unsigned char*>(out);
+#define SB_UPS_LAUNCH(L, VV) \
+  upsample_select_kernel<L, VV><<<grid, 256, 0, stream>>>(planes, P, S, sel, cpp, Ho, Wo, rows, thr, o)
+  if (logits) {
+    switch (V) {
+      case 16: SB_UPS_LAUNCH(true, 16); break;
+      case 8: SB_UPS_LAUNCH(true, 8); break;
+      default: SB_UPS_LAUNCH(true, 4); break;
+    }
+  } else {
+    switch (V) {
+      case 16: SB_UPS_LAUNCH(false, 16); break;
+      case 8: SB_UPS_LAUNCH(false, 8); break;
+      case 4: SB_UPS_LAUNCH(false, 4); break;
+      default: SB_UPS_LAUNCH(false, 1); break;  // odd widths; a 2-byte variant spilled and gained nothing
+    }
+  }
+#undef SB_UPS_LAUNCH
   SB_CHECK_LAUNCH();
   return SB_OK;
 }

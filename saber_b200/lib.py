@@ -95,6 +95,7 @@ SIGNATURES = {
     "sb_resize_normalize": [c_void_p, c_int, c_int, c_int, c_void_p, c_int, c_int, C.POINTER(c_float),
                             C.POINTER(c_float), c_void_p, c_void_p],
     "sb_upsample_bilinear": [c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p],
+    "sb_upsample_select": [c_void_p, c_int, c_int, c_void_p, c_int, c_int, c_int, c_float, c_int, c_void_p, c_void_p],
     "sb_stitch_labels": [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p],
     "sb_ccl3d_26": [c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p],
     "sb_ccl3d": [c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p],

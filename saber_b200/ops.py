@@ -1081,6 +1081,24 @@ def upsample_bilinear(x: torch.Tensor, Ho: int, Wo: int) -> torch.Tensor:
     return out
 
 
+def upsample_select(planes: torch.Tensor, sel: Optional[torch.Tensor], cpp: int, Ho: int, Wo: int,
+                    threshold: float = 0.0, logits: bool = False) -> torch.Tensor:
+    """Decoder planes [P,4,S,S] -> [P, cpp, Ho, Wo] in one kernel: the selected planes (tokens 1..3 for cpp = 3, else the
+    ``sel`` choice or token 0) up-sampled bit-identically to ``upsample_bilinear``, as fp32 logits or as bool
+    ``value > threshold`` masks."""
+    _chk_cuda(planes, sel)
+    assert planes.dtype == _F32 and planes.is_contiguous() and planes.dim() == 4 and planes.shape[1] == 4
+    assert sel is None or (sel.dtype == _I32 and sel.is_contiguous() and sel.numel() == planes.shape[0])
+    assert cpp in (1, 3) and not (cpp == 3 and sel is not None)
+    P, S = planes.shape[0], planes.shape[2]
+    out = torch.empty((P, cpp, Ho, Wo), dtype=_F32 if logits else torch.bool, device=planes.device)
+    L = _lib.load()
+    _lib.check(L.sb_upsample_select(planes.data_ptr(), P, S, _ptr(sel), cpp, Ho, Wo, float(threshold), int(logits),
+                                    out.data_ptr(), _stream()), "sb_upsample_select")
+    _count()
+    return out
+
+
 # ---------------------------------------------------------------------------------------------
 # z-axis propagation: memory attention / memory encoder / tracking glue (csrc/memory.cu)
 # ---------------------------------------------------------------------------------------------
