@@ -290,7 +290,7 @@ __device__ __forceinline__ void epilogue_rows(const GemmParams& p, const EpiSmem
   // 16-byte offsets of this lane's rows (all pitches are multiples of 16 bytes on this path)
   const int res_off16 = (has_res && row_ok) ? static_cast<int>(rrow * p.ldr / (p.res_f32 ? 4 : 8)) : -1;
   const int out_off16 = row_ok ? static_cast<int>(static_cast<long long>(row) * p.ldo / (p.out_f32 ? 4 : 8)) : -1;
-  float sum = 0.f, sumsq = 0.f, mean = 0.f, rstd = 0.f;
+  float sum = 0.f, sumsq = 0.f, shift = 0.f, mean = 0.f, rstd = 0.f;
 #pragma unroll 1
   for (int pass = 0; pass < (LN ? 2 : 1); ++pass) {
     if (n_idx + g_begin * 32 >= p.N) break;
@@ -362,10 +362,14 @@ __device__ __forceinline__ void epilogue_rows(const GemmParams& p, const EpiSmem
         }
         if (LN) {
           if (pass == 0) {
+            // sums of x - x0 (x0 = the row's first value): sumsq / N - mean^2 in fp32 on the raw values loses the
+            // variance of rows whose |mean| is large against their std (rstd off by 2.5e-3 at |mean| / std = 64)
+            if (g == g_begin && h == 0) shift = f[0];
+            const float2 nsh = sb::splat2(-shift);
             float2 s2 = make_float2(0.f, 0.f), q2 = make_float2(0.f, 0.f);
 #pragma unroll
             for (int j = 0; j < CH / 2; ++j) {
-              const float2 ff = make_float2(f[2 * j], f[2 * j + 1]);
+              const float2 ff = sb::add2(make_float2(f[2 * j], f[2 * j + 1]), nsh);
               s2 = sb::add2(s2, ff);
               q2 = sb::fma2(ff, ff, q2);
             }
@@ -411,8 +415,9 @@ __device__ __forceinline__ void epilogue_rows(const GemmParams& p, const EpiSmem
     }
     if (LN && pass == 0) {
       sb::tmem_st_wait();
-      mean = sum / static_cast<float>(p.N);
-      const float var = fmaxf(sumsq / static_cast<float>(p.N) - mean * mean, 0.f);
+      const float dmean = sum / static_cast<float>(p.N);
+      mean = shift + dmean;
+      const float var = fmaxf(sumsq / static_cast<float>(p.N) - dmean * dmean, 0.f);
       rstd = rsqrtf(var + p.eps);
     }
   }

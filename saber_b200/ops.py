@@ -174,6 +174,8 @@ def _gemm_validate(a, w, bias, act, residual, res_mod, out, alpha, force_bn):
     a6 = split3(a, 0)
     if act == ACT_GELU:  # exact erf GELU after the product (the fused MUFU.TANH form is accurate to 4e-4 only)
         assert residual is None
+        # the GELU kernel runs over numel() contiguous elements: a strided `out` would have other elements rewritten
+        assert out is None or out.is_contiguous(), "validation mode: GELU needs a contiguous out"
         y = gemm(a6, w6, bias, ACT_NONE, None, 0, _F32, out=out, alpha=alpha, force_bn=force_bn)
         L = _lib.load()
         _lib.check(L.sb_gelu_exact_f32(y.data_ptr(), y.numel(), _stream()), "sb_gelu_exact_f32")
