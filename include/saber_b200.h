@@ -247,6 +247,12 @@ int sb_upsample_bilinear(const float* in, int N, int Hi, int Wi, int Ho, int Wo,
  * [P*cpp, Ho, Wo]: fp32 logits when logits != 0, else bool (value > thr). out is 16-byte aligned. */
 int sb_upsample_select(const float* planes, int P, int S, const int* sel, int cpp, int Ho, int Wo, float thr,
                        int logits, void* out, void* stream);
+/* Video frames (sam2 load_video_frames): uint8 RGB [N,H,W,3] -> Pillow's 8-bit bicubic resize to S x S -> lut[c][byte]
+ * -> fp32 [N,3,S,S]. x* / y*: per-output (xmin, n) bounds and 22-bit fixed-point weights; x* null skips the horizontal
+ * pass (W == S); tmp: [N,hy,S,3] u8 holding source rows [y0, y0 + hy) after the horizontal pass. */
+int sb_resample_frames_u8(const void* src, int N, int H, int W, int S, const int* xbounds, const int* xweights, int xk,
+                          const int* ybounds, const int* yweights, int yk, int y0, int hy, void* tmp, const float* lut,
+                          float* out, void* stream);
 
 /* ---- z-axis propagation: memory attention / memory encoder / tracking glue (upstream sam2_video_predictor.py, ----
  * modeling/{memory_attention,memory_encoder,sam2_base}.py, reached from REF saber/adapters/sam2/predictor.py:164-202) */

@@ -220,16 +220,9 @@ class SAM2Adapter(BaseAdapter):
 
     def _create_empty_inference_state(self, images, video_height, video_width, offload_video_to_cpu=False,
                                       offload_state_to_cpu=False) -> Dict[str, Any]:
-        """REF :118-154 (same keys)."""
-        from collections import OrderedDict
-        dev = self.device
-        st = {"images": images, "num_frames": len(images), "offload_video_to_cpu": offload_video_to_cpu,
-              "offload_state_to_cpu": offload_state_to_cpu, "video_height": video_height, "video_width": video_width,
-              "device": dev, "storage_device": dev, "point_inputs_per_obj": {}, "mask_inputs_per_obj": {},
-              "cached_features": {}, "constants": {}, "obj_id_to_idx": OrderedDict(), "obj_idx_to_id": OrderedDict(),
-              "obj_ids": [], "output_dict_per_obj": {}, "temp_output_dict_per_obj": {}, "frames_tracked_per_obj": {}}
-        self._video()._get_image_feature(st, frame_idx=0, batch_size=1)
-        return st
+        """REF :118-154 (same keys); the state lives on the adapter's device."""
+        return self._video().new_inference_state(images, video_height, video_width, offload_video_to_cpu,
+                                                 offload_state_to_cpu, self.device, self.device)
 
     def add_new_mask(self, frame_idx: int, obj_id: int, mask, inference_state=None):
         state = inference_state or self.inference_state

@@ -96,6 +96,8 @@ SIGNATURES = {
                             C.POINTER(c_float), c_void_p, c_void_p],
     "sb_upsample_bilinear": [c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p],
     "sb_upsample_select": [c_void_p, c_int, c_int, c_void_p, c_int, c_int, c_int, c_float, c_int, c_void_p, c_void_p],
+    "sb_resample_frames_u8": [c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_int,
+                              c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p],
     "sb_stitch_labels": [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p],
     "sb_ccl3d_26": [c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p],
     "sb_ccl3d": [c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p],

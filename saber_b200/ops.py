@@ -1101,6 +1101,76 @@ def upsample_select(planes: torch.Tensor, sel: Optional[torch.Tensor], cpp: int,
     return out
 
 
+_frame_coeff_cache: dict = {}
+
+
+def pillow_bicubic_coeffs(n_in: int, n_out: int):
+    """Pillow's 8-bit BICUBIC coefficients (libImaging/Resample.c precompute_coeffs + normalize_coeffs_8bpc) in float64
+    with Pillow's order of operations -> (bounds int32 [n_out, 2] = (xmin, n), weights int32 [n_out, ksize])."""
+    import numpy as np
+    scale = n_in / n_out
+    fs = max(scale, 1.0)
+    support = 2.0 * fs
+    ksize = int(math.ceil(support)) * 2 + 1
+    center = (np.arange(n_out, dtype=np.float64) + 0.5) * scale
+    xmin = np.maximum((center - support + 0.5).astype(np.int64), 0)  # C (int) truncates toward zero, as astype does
+    n = np.minimum((center + support + 0.5).astype(np.int64), n_in) - xmin
+    k = np.arange(ksize)
+    t = np.abs((k[None, :] + xmin[:, None] - center[:, None] + 0.5) * (1.0 / fs))
+    a = -0.5
+    w = np.where(t < 1.0, ((a + 2.0) * t - (a + 3.0)) * t * t + 1,
+                 np.where(t < 2.0, (((t - 5) * t + 8) * t - 4) * a, 0.0))
+    w = np.where(k[None, :] < n[:, None], w, 0.0)
+    ww = np.zeros(n_out)
+    for j in range(ksize):  # Pillow sums the taps in order (numpy's pairwise sum would round differently)
+        ww = ww + w[:, j]
+    w = np.where(ww[:, None] != 0.0, w / np.where(ww == 0.0, 1.0, ww)[:, None], w)
+    fixed = np.where(w < 0, -0.5 + w * (1 << 22), 0.5 + w * (1 << 22)).astype(np.int64)
+    return np.stack([xmin, n], 1).astype(np.int32), fixed.astype(np.int32)
+
+
+def _frame_coeffs(n_in: int, n_out: int, device):
+    """Device coefficient tables of one axis, cached per (n_in, n_out, device): (bounds, weights, ksize, first, last),
+    with [first, last) the source range the taps reach. n_in == n_out gives the one-tap identity (pass skipped)."""
+    key = (n_in, n_out, str(device))
+    c = _frame_coeff_cache.get(key)
+    if c is None:
+        import numpy as np
+        if n_in == n_out:
+            b = np.stack([np.arange(n_out), np.ones(n_out, np.int64)], 1).astype(np.int32)
+            w = np.full((n_out, 1), 1 << 22, np.int32)
+        else:
+            b, w = pillow_bicubic_coeffs(n_in, n_out)
+        c = (torch.from_numpy(b).to(device), torch.from_numpy(np.ascontiguousarray(w)).to(device), w.shape[1],
+             int(b[0, 0]), int(b[-1, 0] + b[-1, 1]))
+        _frame_coeff_cache[key] = c
+    return c
+
+
+def resample_frames_u8(frames: torch.Tensor, S: int, lut: torch.Tensor, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """uint8 RGB frames [N, H, W, 3] of one size -> fp32 [N, 3, S, S]: Pillow's ``Image.resize((S, S))`` (bicubic,
+    8-bit fixed point) bit for bit, then ``lut[c, byte]`` ([3, 256] fp32). ``out``: optional contiguous destination."""
+    _chk_cuda(frames, lut, out)
+    assert frames.dtype == torch.uint8 and frames.is_contiguous() and frames.dim() == 4 and frames.shape[3] == 3
+    assert lut.dtype == _F32 and lut.is_contiguous() and lut.numel() == 3 * 256
+    N, H, W, _ = frames.shape
+    if out is None:
+        out = torch.empty((N, 3, S, S), dtype=_F32, device=frames.device)
+    assert out.dtype == _F32 and out.is_contiguous() and tuple(out.shape) == (N, 3, S, S)
+    yb, yw, yk, y0, y1 = _frame_coeffs(H, S, frames.device)
+    xb = xw = tmp = None
+    xk = 0
+    if W != S:
+        xb, xw, xk, _, _ = _frame_coeffs(W, S, frames.device)
+        tmp = torch.empty((N, y1 - y0, S, 3), dtype=torch.uint8, device=frames.device)
+    L = _lib.load()
+    _lib.check(L.sb_resample_frames_u8(frames.data_ptr(), N, H, W, S, _ptr(xb), _ptr(xw), xk, yb.data_ptr(), yw.data_ptr(),
+                                       yk, y0, y1 - y0, _ptr(tmp), lut.data_ptr(), out.data_ptr(), _stream()),
+               "sb_resample_frames_u8")
+    _count(2 if tmp is not None else 1)
+    return out
+
+
 # ---------------------------------------------------------------------------------------------
 # z-axis propagation: memory attention / memory encoder / tracking glue (csrc/memory.cu)
 # ---------------------------------------------------------------------------------------------

@@ -515,6 +515,33 @@ class SAM2VideoPredictor(SAM2Model):
             yield frame_idx, obj_ids, video_res
 
     # ---- state ------------------------------------------------------------------------------------------------
+    @torch.inference_mode()
+    def init_state(self, video_path, offload_video_to_cpu=False, offload_state_to_cpu=False, async_loading_frames=False):
+        """Upstream's ``init_state`` on a folder of JPEG frames (``video_io.load_video_frames``): the inference-state
+        dict with frame 0's features warmed. ``storage_device`` is the host with ``offload_state_to_cpu``, as upstream
+        reports it; the memory bank stays on the device either way (the outputs do not depend on it)."""
+        from .video_io import load_video_frames
+        self._require_gpu()
+        images, video_height, video_width = load_video_frames(video_path, self.image_size, offload_video_to_cpu,
+                                                              async_loading_frames=async_loading_frames,
+                                                              compute_device=self.device)
+        storage = torch.device("cpu") if offload_state_to_cpu else self.device
+        return self.new_inference_state(images, video_height, video_width, offload_video_to_cpu, offload_state_to_cpu,
+                                        self.device, storage)
+
+    def new_inference_state(self, images, video_height, video_width, offload_video_to_cpu, offload_state_to_cpu,
+                            device, storage_device) -> Dict[str, Any]:
+        """Upstream's inference-state dict (same keys, same value types) over ``images`` [N,3,S,S] or a lazy frame
+        list, with frame 0's features warmed through ``_get_image_feature`` as upstream's ``init_state`` does."""
+        from collections import OrderedDict
+        st = {"images": images, "num_frames": len(images), "offload_video_to_cpu": offload_video_to_cpu,
+              "offload_state_to_cpu": offload_state_to_cpu, "video_height": video_height, "video_width": video_width,
+              "device": device, "storage_device": storage_device, "point_inputs_per_obj": {}, "mask_inputs_per_obj": {},
+              "cached_features": {}, "constants": {}, "obj_id_to_idx": OrderedDict(), "obj_idx_to_id": OrderedDict(),
+              "obj_ids": [], "output_dict_per_obj": {}, "temp_output_dict_per_obj": {}, "frames_tracked_per_obj": {}}
+        self._get_image_feature(st, frame_idx=0, batch_size=1)
+        return st
+
     @torch.no_grad()
     def reset_state(self, inference_state):
         s = inference_state
