@@ -157,10 +157,6 @@ int sb_mask_downscale(const float* in, int B, int S, int cpp, float clampv, cons
  * keys[b*T+t] = bf16(image_embed[t] + bias + ds[b*T+t] @ w^T); ds [ntok,16] bf16, w [256,16] fp32, image_embed [T,256] */
 int sb_mask_embed_keys(const void* ds, const float* w, const float* bias, const float* image_embed, int T, long long ntok,
                        void* keys, void* stream);
-int sb_upscale1_post(const void* g1, const float* feat_s1, long long s1_batch_stride, const float* gamma,
-                     const float* beta, int B, int h, int w, void* u1, void* stream);
-int sb_upscale2_mask(const void* g2, const float* feat_s0, long long s0_batch_stride, const float* hyper, int B,
-                     int H1, int W1, float* masks, void* stream);
 /* MaskDecoder._dynamic_multimask_via_stability (delta 0.05, thresh 0.98 set by build_sam2(apply_postprocessing)) */
 int sb_select_mask(const float* masks, const float* ious, int B, int HW, float delta, float thresh, int* sel_idx,
                    float* sel_iou, void* stream);

@@ -1,8 +1,8 @@
 // saber_b200 — SAM2 prompt-encoder / mask-decoder glue kernels (everything that is not a GEMM,
 // LayerNorm or attention): point-prompt token assembly with random-Fourier positional encoding,
-// the fused mask-prompt down-scaling convs, the two transposed-conv post stages (pixel shuffle +
-// skip + LayerNorm2d + GELU, and pixel shuffle + skip + GELU + hyper-network mask product), and the
-// dynamic-multimask-via-stability selection.
+// the fused mask-prompt down-scaling convs, the m2m pass's per-prompt image stream, the IoU gate and
+// the dynamic-multimask-via-stability selection. (The transposed-conv up-scaling stages are fused
+// into the GEMM epilogues of gemm_tcgen05.cu.)
 // Restates sam2/modeling/sam/prompt_encoder.py and mask_decoder.py (SURVEY §8a U2/U3; HF
 // modeling_sam2.py:712-856, 859-1296) as called from REF saber/adapters/sam2/automask.py:66-78.
 #include "common.cuh"
@@ -220,80 +220,6 @@ mask_embed_keys_kernel(const __nv_bfloat16* __restrict__ ds, const float* __rest
   }
 }
 
-// Stage 1 of output_upscaling after the ConvTranspose2d(256->64,k2,s2) GEMM:
-// g1 [B*h*w, 4*64] (col = (dy*2+dx)*64 + co, bias included) -> pixel shuffle -> + feat_s1 ->
-// LayerNorm2d(64) -> GELU -> u1 [B*(2h)*(2w), 64] bf16. One warp per (token, dydx).
-__global__ void __launch_bounds__(256)
-upscale1_post_kernel(const __nv_bfloat16* __restrict__ g1, const float* __restrict__ feat_s1,
-                     const float* __restrict__ gamma, const float* __restrict__ beta, int B, int h,
-                     int w, long long s1_batch_stride, __nv_bfloat16* __restrict__ u1) {
-  const int lane = threadIdx.x & 31;
-  const long long nwarp_total = static_cast<long long>(B) * h * w * 4;
-  const float g0 = gamma[2 * lane], g1v = gamma[2 * lane + 1];
-  const float b0 = beta[2 * lane], b1v = beta[2 * lane + 1];
-  for (long long wi = (static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x) >> 5;
-       wi < nwarp_total; wi += (static_cast<long long>(gridDim.x) * blockDim.x) >> 5) {
-    const int d = static_cast<int>(wi & 3);
-    const long long tok = wi >> 2;
-    const int x = static_cast<int>(tok % w), y = static_cast<int>((tok / w) % h);
-    const long long b = tok / (static_cast<long long>(w) * h);
-    const int oy = 2 * y + (d >> 1), ox = 2 * x + (d & 1);
-    const uint32_t gv = *reinterpret_cast<const uint32_t*>(g1 + tok * 256 + d * 64 + 2 * lane);
-    const float2 sv = *reinterpret_cast<const float2*>(
-        feat_s1 + b * s1_batch_stride + (static_cast<long long>(oy) * (2 * w) + ox) * 64 + 2 * lane);
-    const float v0 = sb::bf16_lo(gv) + sv.x, v1 = sb::bf16_hi(gv) + sv.y;
-    const float mean = sb::warp_sum(v0 + v1) * (1.f / 64.f);
-    const float d0 = v0 - mean, d1 = v1 - mean;
-    const float rstd = rsqrtf(sb::warp_sum(d0 * d0 + d1 * d1) * (1.f / 64.f) + 1e-6f);
-    const float o0 = sb::gelu_erf(d0 * rstd * g0 + b0), o1 = sb::gelu_erf(d1 * rstd * g1v + b1v);
-    *reinterpret_cast<uint32_t*>(u1 + ((b * (2 * h) + oy) * (2 * w) + ox) * 64 + 2 * lane) =
-        sb::pack_bf16x2(o0, o1);
-  }
-}
-
-// Stage 2: g2 [B*H1*W1, 4*32] (col = (dy*2+dx)*32 + co, bias included) -> pixel shuffle -> + feat_s0
-// -> GELU -> dot with hyper_in[b, m, 0..31] -> masks [B, 4, 2*H1, 2*W1] fp32. One warp per token:
-// lane = dydx*8 + cg handles 4 channels of one of the 4 output pixels.
-__global__ void __launch_bounds__(256)
-upscale2_mask_kernel(const __nv_bfloat16* __restrict__ g2, const float* __restrict__ feat_s0,
-                     const float* __restrict__ hyper, int B, int H1, int W1,
-                     long long s0_batch_stride, float* __restrict__ masks) {
-  const int lane = threadIdx.x & 31;
-  const int d = lane >> 3, cg = lane & 7;
-  const long long ntok = static_cast<long long>(B) * H1 * W1;
-  const int H2 = 2 * H1, W2 = 2 * W1;
-  for (long long tok = (static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x) >> 5; tok < ntok;
-       tok += (static_cast<long long>(gridDim.x) * blockDim.x) >> 5) {
-    const int x = static_cast<int>(tok % W1), y = static_cast<int>((tok / W1) % H1);
-    const long long b = tok / (static_cast<long long>(W1) * H1);
-    const int oy = 2 * y + (d >> 1), ox = 2 * x + (d & 1);
-    const uint2 gv = *reinterpret_cast<const uint2*>(g2 + tok * 128 + d * 32 + cg * 4);
-    const float4 sv = *reinterpret_cast<const float4*>(
-        feat_s0 + b * s0_batch_stride + (static_cast<long long>(oy) * W2 + ox) * 32 + cg * 4);
-    const float v0 = sb::gelu_erf(sb::bf16_lo(gv.x) + sv.x);
-    const float v1 = sb::gelu_erf(sb::bf16_hi(gv.x) + sv.y);
-    const float v2 = sb::gelu_erf(sb::bf16_lo(gv.y) + sv.z);
-    const float v3 = sb::gelu_erf(sb::bf16_hi(gv.y) + sv.w);
-    float acc[4];
-#pragma unroll
-    for (int m = 0; m < 4; ++m) {
-      const float4 hv = *reinterpret_cast<const float4*>(hyper + (b * 4 + m) * 32 + cg * 4);
-      acc[m] = v0 * hv.x + v1 * hv.y + v2 * hv.z + v3 * hv.w;
-    }
-#pragma unroll
-    for (int m = 0; m < 4; ++m) {
-      acc[m] += __shfl_xor_sync(0xffffffffu, acc[m], 1);
-      acc[m] += __shfl_xor_sync(0xffffffffu, acc[m], 2);
-      acc[m] += __shfl_xor_sync(0xffffffffu, acc[m], 4);
-    }
-    if (cg < 4) {
-      // lanes cg=0..3 of each pixel group store mask m = cg
-      const float val = cg == 0 ? acc[0] : (cg == 1 ? acc[1] : (cg == 2 ? acc[2] : acc[3]));
-      masks[((b * 4 + cg) * H2 + oy) * W2 + ox] = val;
-    }
-  }
-}
-
 // AMG m2m pass: which prompts can still pass `iou > thresh` whatever dynamic_multimask_via_stability picks? The output
 // IoU of a prompt is ious[b][0] or max(ious[b][1..3]), so max over the four is an upper bound: prompts below it are
 // discarded by SAM2AutomaticMaskGenerator's pred_iou_thresh filter without their masks ever being looked at
@@ -443,31 +369,6 @@ extern "C" int sb_mask_embed_keys(const void* ds, const float* w, const float* b
   dim3 grid((T / 16 + 3) / 4, (nprompts + MEK_PPW - 1) / MEK_PPW);
   mask_embed_keys_kernel<<<grid, 128, 0, stream>>>(
       static_cast<const __nv_bfloat16*>(ds), w, bias, image_embed, T, nprompts, static_cast<__nv_bfloat16*>(keys));
-  SB_CHECK_LAUNCH();
-  return SB_OK;
-}
-
-extern "C" int sb_upscale1_post(const void* g1, const float* feat_s1, long long s1_batch_stride,
-                                const float* gamma, const float* beta, int B, int h, int w, void* u1,
-                                void* stream_) {
-  cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
-  SB_REQUIRE(B > 0 && h > 0 && w > 0, "sb_upscale1_post: bad sizes");
-  const long long threads = static_cast<long long>(B) * h * w * 4 * 32;
-  upscale1_post_kernel<<<blocks_for(threads, 256, 148 * 32), 256, 0, stream>>>(
-      static_cast<const __nv_bfloat16*>(g1), feat_s1, gamma, beta, B, h, w, s1_batch_stride,
-      static_cast<__nv_bfloat16*>(u1));
-  SB_CHECK_LAUNCH();
-  return SB_OK;
-}
-
-extern "C" int sb_upscale2_mask(const void* g2, const float* feat_s0, long long s0_batch_stride,
-                                const float* hyper, int B, int H1, int W1, float* masks,
-                                void* stream_) {
-  cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
-  SB_REQUIRE(B > 0 && H1 > 0 && W1 > 0, "sb_upscale2_mask: bad sizes");
-  const long long threads = static_cast<long long>(B) * H1 * W1 * 32;
-  upscale2_mask_kernel<<<blocks_for(threads, 256, 148 * 32), 256, 0, stream>>>(
-      static_cast<const __nv_bfloat16*>(g2), feat_s0, hyper, B, H1, W1, s0_batch_stride, masks);
   SB_CHECK_LAUNCH();
   return SB_OK;
 }

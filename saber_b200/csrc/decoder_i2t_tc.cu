@@ -9,7 +9,8 @@
 //     P = per-head softmax(S)    (one thread per (row, column half); written to shared memory as the K-major,
 //                                  128B-swizzled A operand of the second MMA)
 //     O = P W2                   (tcgen05.mma M128 N256 K64, accumulator in TMEM)
-//     keys_new = LN(X + O)       (two passes over TMEM; the residual is read from the TMA-staged X tile)
+//     keys_new = LN(X + O)       (two passes over TMEM; the residual is read from the TMA-staged X tile; the row
+//                                  statistics are sums of y - x0, x0 = the row's first residual value)
 // Both GEMMs run on the tensor core so that W1 / W2 are read once per 128-row tile (an earlier mma.sync kernel re-read
 // them from shared memory for every 16 rows and was shared-memory / latency bound at ~2.2 TB/s of HBM traffic); the
 // SM's LSU bandwidth is left to the softmax / LayerNorm epilogue.
@@ -250,27 +251,37 @@ i2t_tc_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ C
       sb::tmem_ld_32x16(ta, v);
       sb::tmem_ld_32x16(ta + 16, v + 16);
       sb::tmem_ld_wait();
-      // ---- per-head softmax over the 8 token slots; P as bf16, one 16-byte chunk per head
+      // ---- per-head softmax over the 8 token slots; P as bf16, one 16-byte chunk per head. The elementwise steps run
+      // on packed pairs (the same IEEE operations as the scalar form); the row sum stays in slot order.
 #pragma unroll
       for (int j = 0; j < 4; ++j) {
-        float s[8];
+        float2 s[4];
         float mx = -INFINITY;
 #pragma unroll
-        for (int t = 0; t < 8; ++t) {
-          s[t] = t < nt ? __uint_as_float(v[j * 8 + t]) + pe[j * 8 + t] : -INFINITY;
-          mx = fmaxf(mx, s[t]);
+        for (int u = 0; u < 4; ++u) {
+          s[u] = sb::add2(make_float2(__uint_as_float(v[j * 8 + 2 * u]), __uint_as_float(v[j * 8 + 2 * u + 1])),
+                          make_float2(pe[j * 8 + 2 * u], pe[j * 8 + 2 * u + 1]));
+          if (2 * u >= nt) s[u].x = -INFINITY;
+          if (2 * u + 1 >= nt) s[u].y = -INFINITY;
+          mx = fmaxf(mx, fmaxf(s[u].x, s[u].y));
         }
         float l = 0.f;
 #pragma unroll
-        for (int t = 0; t < 8; ++t) {
-          s[t] = sb::fast_exp2(s[t] - mx);
-          l += s[t];
+        for (int u = 0; u < 4; ++u) {
+          s[u] = sb::add2(s[u], sb::splat2(-mx));
+          s[u] = make_float2(sb::fast_exp2(s[u].x), sb::fast_exp2(s[u].y));
+          l += s[u].x;
+          l += s[u].y;
         }
-        const float inv = __fdividef(1.f, l);
+        const float2 inv = sb::splat2(__fdividef(1.f, l));
         const int chunk = hf * 4 + j;
-        sts128(sbase + TC_OFF_P + r * 128 + ((chunk ^ (r & 7)) << 4),
-               make_uint4(sb::pack_bf16x2(s[0] * inv, s[1] * inv), sb::pack_bf16x2(s[2] * inv, s[3] * inv),
-                          sb::pack_bf16x2(s[4] * inv, s[5] * inv), sb::pack_bf16x2(s[6] * inv, s[7] * inv)));
+        uint32_t pk[4];
+#pragma unroll
+        for (int u = 0; u < 4; ++u) {
+          const float2 pp = sb::mul2(s[u], inv);
+          pk[u] = sb::pack_bf16x2(pp.x, pp.y);
+        }
+        sts128(sbase + TC_OFF_P + r * 128 + ((chunk ^ (r & 7)) << 4), make_uint4(pk[0], pk[1], pk[2], pk[3]));
       }
       sb::tc_fence_before();
       sb::fence_proxy_async();  // P (generic-proxy stores) -> visible to the tensor core's async-proxy reads
@@ -288,6 +299,11 @@ i2t_tc_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ C
       sb::mbar_wait(&o_full[buf], static_cast<uint32_t>((n >> 1) & 1));
       sb::tc_fence_after();
       sb::mbar_wait(&x_full[buf], static_cast<uint32_t>((n >> 1) & 1));  // (already complete) TMA writes -> this thread
+      // d = y - x0 (x0 = column 0 of the row in the staged X tile, read by both column halves) is what is summed and
+      // parked in TMEM: a one-pass variance of the raw y (sumsq / 256 - mean^2) cancels catastrophically on rows whose
+      // |mean| / std is in the hundreds
+      const float x0 = sb::bf16_lo(lds128(sbase + buf * TC_XBUF + r * 128 + ((r & 7) << 4)).x);
+      const float2 nx0 = make_float2(-x0, -x0);
       float2 sum2 = make_float2(0.f, 0.f), sq2 = make_float2(0.f, 0.f);
 #pragma unroll 1
       for (int c = 0; c < 4; ++c) {
@@ -305,8 +321,8 @@ i2t_tc_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ C
           const uint32_t w4[4] = {res[j].x, res[j].y, res[j].z, res[j].w};
 #pragma unroll
           for (int e = 0; e < 4; ++e) {
-            const float2 yy = sb::add2(make_float2(__uint_as_float(v[8 * j + 2 * e]), __uint_as_float(v[8 * j + 2 * e + 1])),
-                                   make_float2(sb::bf16_lo(w4[e]), sb::bf16_hi(w4[e])));
+            const float2 yy = sb::add2(sb::add2(make_float2(__uint_as_float(v[8 * j + 2 * e]), __uint_as_float(v[8 * j + 2 * e + 1])),
+                                                make_float2(sb::bf16_lo(w4[e]), sb::bf16_hi(w4[e]))), nx0);
             y[8 * j + 2 * e] = yy.x;
             y[8 * j + 2 * e + 1] = yy.y;
             sum2 = sb::add2(sum2, yy);
@@ -330,7 +346,7 @@ i2t_tc_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ C
         sumsq += pq;
       }
       pair_barrier(q);  // both warps have read before the tiles are reused
-      mean = sum * (1.f / 256.f);
+      mean = sum * (1.f / 256.f);  // of d
       rstd = rsqrtf(fmaxf(sumsq * (1.f / 256.f) - mean * mean, 0.f) + p.eps);
 
       // ---------------- S(n+1): softmax of the next tile (its first MMA ran under LN1) ----------------
@@ -348,15 +364,18 @@ i2t_tc_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ C
         const float* ga = sVec + hf * 128 + c * 32;
         const float* be = sVec + 256 + hf * 128 + c * 32;
         uint32_t o16[16];
-        const float2 rs2 = make_float2(rstd, rstd), nm2 = make_float2(-mean, -mean);
+        // (d - mean) * rstd = fma(d, rstd, -mean * rstd): d and mean are sums of y - x0, a few std at most, so the
+        // rounding of -mean * rstd stays at ~2^-24; then * gamma + beta. Two packed instructions per pair of columns,
+        // one fewer than the shift costs in LN1.
+        const float2 rs2 = make_float2(rstd, rstd), nmr2 = make_float2(-mean * rstd, -mean * rstd);
 #pragma unroll
         for (int j = 0; j < 8; ++j) {
           const float4 g4 = *reinterpret_cast<const float4*>(ga + 4 * j);
           const float4 b4 = *reinterpret_cast<const float4*>(be + 4 * j);
-          const float2 d0 = sb::add2(make_float2(__uint_as_float(v[4 * j + 0]), __uint_as_float(v[4 * j + 1])), nm2);
-          const float2 d1 = sb::add2(make_float2(__uint_as_float(v[4 * j + 2]), __uint_as_float(v[4 * j + 3])), nm2);
-          const float2 f01 = sb::fma2(d0, sb::mul2(rs2, make_float2(g4.x, g4.y)), make_float2(b4.x, b4.y));
-          const float2 f23 = sb::fma2(d1, sb::mul2(rs2, make_float2(g4.z, g4.w)), make_float2(b4.z, b4.w));
+          const float2 z0 = sb::fma2(make_float2(__uint_as_float(v[4 * j + 0]), __uint_as_float(v[4 * j + 1])), rs2, nmr2);
+          const float2 z1 = sb::fma2(make_float2(__uint_as_float(v[4 * j + 2]), __uint_as_float(v[4 * j + 3])), rs2, nmr2);
+          const float2 f01 = sb::fma2(z0, make_float2(g4.x, g4.y), make_float2(b4.x, b4.y));
+          const float2 f23 = sb::fma2(z1, make_float2(g4.z, g4.w), make_float2(b4.z, b4.w));
           o16[2 * j] = sb::pack_bf16x2(f01.x, f01.y);
           o16[2 * j + 1] = sb::pack_bf16x2(f23.x, f23.y);
         }

@@ -67,9 +67,6 @@ SIGNATURES = {
                          c_int, c_void_p, c_void_p],
     "sb_mask_downscale": [c_void_p, c_int, c_int, c_int, c_float, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                           c_void_p, c_void_p, c_void_p, c_void_p, c_void_p],
-    "sb_upscale1_post": [c_void_p, c_void_p, c_ll, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p,
-                         c_void_p],
-    "sb_upscale2_mask": [c_void_p, c_void_p, c_ll, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p],
     "sb_select_mask": [c_void_p, c_void_p, c_int, c_int, c_float, c_float, c_void_p, c_void_p, c_void_p],
     "sb_amg_mask_post": [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int,
                          c_int, c_float, c_float, c_float, c_float, c_void_p, c_void_p, c_void_p, c_void_p,

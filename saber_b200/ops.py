@@ -509,7 +509,9 @@ def t2i_fold_attention(q: torch.Tensor, x: torch.Tensor, kadd: torch.Tensor, wk:
 
 
 def mask_embed_keys(ds: torch.Tensor, w: torch.Tensor, bias: torch.Tensor, image_embed: torch.Tensor) -> torch.Tensor:
-    """Per-prompt image stream of the m2m pass: bf16(image_embed[t] + bias + ds @ w^T); ds [B*T,16] bf16, w [256,16] fp32."""
+    """Per-prompt image stream of the m2m pass: bf16(image_embed[t] + bias + ds @ w^T); ds [B*T,16] bf16, w [256,16] fp32.
+    The kernel rounds ``w`` to bf16 (the product is one bf16 tensor-core step per 16 tokens) and accumulates in fp32 from
+    ``image_embed + bias``, so the result is that of the bf16-rounded ``w``, not of the fp32 one."""
     _chk_cuda(ds, w, bias, image_embed)
     assert ds.dtype == _BF16 and ds.is_contiguous() and ds.shape[1] == 16 and w.dtype == _F32 and w.shape == (256, 16)
     assert image_embed.dtype == _F32 and image_embed.is_contiguous() and image_embed.shape[1] == 256
@@ -695,33 +697,6 @@ def mask_downscale(mask: torch.Tensor, w, clamp: float = 0.0) -> torch.Tensor:
                                    _stream()), "sb_mask_downscale")
     _count()
     return out
-
-
-def upscale1_post(g1: torch.Tensor, feat_s1: torch.Tensor, s1_batch_stride: int, gamma: torch.Tensor,
-                  beta: torch.Tensor, B: int, h: int, w: int) -> torch.Tensor:
-    _chk_cuda(g1, feat_s1, gamma, beta)
-    assert g1.dtype == _BF16 and g1.is_contiguous() and g1.shape == (B * h * w, 256)
-    assert feat_s1.dtype == _F32 and feat_s1.is_contiguous()
-    u1 = torch.empty((B * 4 * h * w, 64), dtype=_BF16, device=g1.device)
-    L = _lib.load()
-    _lib.check(L.sb_upscale1_post(g1.data_ptr(), feat_s1.data_ptr(), s1_batch_stride, gamma.data_ptr(),
-                                  beta.data_ptr(), B, h, w, u1.data_ptr(), _stream()), "sb_upscale1_post")
-    _count()
-    return u1
-
-
-def upscale2_mask(g2: torch.Tensor, feat_s0: torch.Tensor, s0_batch_stride: int, hyper: torch.Tensor, B: int,
-                  H1: int, W1: int) -> torch.Tensor:
-    _chk_cuda(g2, feat_s0, hyper)
-    assert g2.dtype == _BF16 and g2.is_contiguous() and g2.shape == (B * H1 * W1, 128)
-    assert feat_s0.dtype == _F32 and feat_s0.is_contiguous()
-    assert hyper.dtype == _F32 and hyper.is_contiguous() and hyper.shape == (B, 4, 32)
-    masks = torch.empty((B, 4, 2 * H1, 2 * W1), dtype=_F32, device=g2.device)
-    L = _lib.load()
-    _lib.check(L.sb_upscale2_mask(g2.data_ptr(), feat_s0.data_ptr(), s0_batch_stride, hyper.data_ptr(), B, H1, W1,
-                                  masks.data_ptr(), _stream()), "sb_upscale2_mask")
-    _count()
-    return masks
 
 
 def select_mask(masks: torch.Tensor, ious: torch.Tensor, delta: float, thresh: float):
